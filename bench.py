@@ -17,6 +17,10 @@ poses of all timed steps are all-gathered over NCCL ONCE, at the end of the time
 Other BASELINE configs: `--frames-per-gpu B` / `--global-frames B` (configs[2] sweep; `--sweep a,b,c` runs several
 totals in one process, one JSON line each), `--volume-size 128` (configs[3]), `--graph` (CUDA-graph lift for the
 batch-1 demo.py case), tools/microbench_geometry.py (configs[4]).
+
+`--dump-outputs DIR` writes the 4-tuple that the last timed step returned (keypoints_3d, features, volumes,
+coord_volumes) as DIR/<name>.npy in float32, so that two builds can be compared output for output on identical
+seeded inputs.  An output larger than DUMP_SAMPLE elements is written as a fixed, seeded sample of its elements.
 """
 import argparse
 import json
@@ -35,6 +39,7 @@ FRAMES_PER_GPU = 64
 J = 15
 FEATURES_BYTES_PER_FRAME = 32 * 1024 * 1280 * 4            # output #2 of the reference forward
 FEATURES_BUDGET_BYTES = 100e9                              # above this, output #2 is not materialised (says so)
+DUMP_SAMPLE = 1 << 21                                      # --dump-outputs: at most 8 MB per output, 32 MB in all
 
 
 def parse():
@@ -62,7 +67,12 @@ def parse():
                     help="storage type of V2V activations / weights (bf16 = BASELINE configs[1]; f16 = the fp16 build)")
     ap.add_argument("--profile-ops", default="", help="write the per-op V2V timing table to this file")
     ap.add_argument("--out", default="", help="also append the JSON line(s) to this file")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0's frames) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def workload_config(frames, world, V=64, chunk=64, strong=False, features=True, graph=False):
@@ -88,6 +98,22 @@ def emit(line, args):
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "a") as f:
             f.write(s + "\n")
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output tensor (None: not materialised, skipped) as out_dir/<name>.npy in float32.  One with more
+    than DUMP_SAMPLE elements is written flat, as its elements at DUMP_SAMPLE ascending flat indices drawn from a
+    CPU generator seeded with 0: the same indices in every run with the same arguments."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        if t is None:
+            continue
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 # --------------------------------------------------------------------------------------
@@ -343,11 +369,16 @@ def run_config(args, net, B, total, world, rank, local, dev, V, strong, features
     feat_d, depth_d = feat_h.to(dev), depth_h.to(dev)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev) if B < 16 else None
 
-    def step():
+    last = {}
+
+    def step(keep=False):
         if flush is not None:
             flush.zero_()                     # small batches fit the 126 MB L2: flush it between timed steps
         with torch.no_grad():
-            return net.lift(feat_d, net.grid_coord_proj_batch, net.coord_volumes, depth_map_batch=depth_d)[0]
+            out = net.lift(feat_d, net.grid_coord_proj_batch, net.coord_volumes, depth_map_batch=depth_d)
+        if keep:
+            last.update(zip(("keypoints_3d", "features", "volumes", "coord_volumes"), out))
+        return out[0]
 
     def barrier():
         if world > 1:
@@ -367,8 +398,8 @@ def run_config(args, net, B, total, world, rank, local, dev, V, strong, features
     e0.record()
     launches = 0
     kps = []
-    for _ in range(args.steps):
-        kps.append(step())
+    for i in range(args.steps):
+        kps.append(step(keep=bool(args.dump_outputs) and i == args.steps - 1))
         launches += net.last_launches
     all_kp = torch.stack(kps)                              # (steps, B, J, 3)
     if world > 1:                                          # the ONE collective: final gather of the poses
@@ -391,6 +422,9 @@ def run_config(args, net, B, total, world, rank, local, dev, V, strong, features
     clocks = sampler.window(t_wall0, t_wall1) if rank == 0 else None
     value = total * args.steps / (ms_total / 1000.0)
     assert torch.isfinite(all_kp).all()
+    if last and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
 
     # ---- end to end: pinned host buffers -> H2D -> lift -> D2H, through the public pipeline ----
     if args.raw_depth:

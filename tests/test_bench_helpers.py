@@ -4,6 +4,10 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+import torch
+
 from tests import util
 
 sys.path.insert(0, util.ROOT)
@@ -42,3 +46,39 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
         assert k in d, k
     assert d["impl"] == "reference" and d["frames_run_per_step"] == 1 and d["cpu_baseline"]["kind"] == "port"
     assert d["config"] == bench.workload_config(64, 1, 64, 64) and d["value"] > 0 and d["e2e"]["h2d_bytes_per_step"] == 0
+
+
+def test_dump_outputs_writes_float32_and_a_fixed_sample(tmp_path, monkeypatch):
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 100)
+    kp = torch.randn(2, 15, 3)
+    big = torch.arange(1000, dtype=torch.float64).reshape(10, 100)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"keypoints_3d": kp, "features": None, "volumes": big})
+    assert sorted(os.listdir(tmp_path / "a")) == ["keypoints_3d.npy", "volumes.npy"]
+    k = np.load(tmp_path / "a" / "keypoints_3d.npy")
+    assert k.dtype == np.float32 and np.array_equal(k, kp.numpy())             # small outputs: whole, shape kept
+    va, vb = np.load(tmp_path / "a" / "volumes.npy"), np.load(tmp_path / "b" / "volumes.npy")
+    assert va.dtype == np.float32 and va.shape == (100,) and np.array_equal(va, vb)
+    assert np.all(np.diff(va) >= 0) and len(np.unique(va)) > 50                # ascending flat indices, spread out
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_same_outputs_from_run_to_run(tmp_path):
+    """`bench.py --dump-outputs` twice with the same arguments: the last timed step's outputs agree bit for bit."""
+    for d in ("a", "b"):
+        r = subprocess.run([sys.executable, "bench.py", "--steps", "2", "--warmup", "0", "--frames-per-gpu", "2",
+                            "--no-kernel-table", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / d)],
+                           cwd=util.ROOT, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-1500:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 2
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["coord_volumes.npy", "features.npy", "keypoints_3d.npy", "volumes.npy"]
+    total = 0
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float32 and np.array_equal(a, b), n
+        total += a.nbytes
+    assert total <= 64 << 20
+    kp = np.load(tmp_path / "a" / "keypoints_3d.npy")
+    assert kp.shape == (2, 15, 3) and np.isfinite(kp).all()
