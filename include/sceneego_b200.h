@@ -184,6 +184,20 @@ int sceneego_voxelize_depth_dataset_f64(const float* d_depth_raw, int batch, int
                                         float clamp_max, const double* d_ray, int volume_size, double cuboid_side,
                                         float* d_occ_f32, void* stream);
 
+/* point_cloud_to_voxel_numpy (network/voxel_net_depth.py:207-222) and point_cloud_to_voxel_pytorch
+ * (dataset/real_depth_utils.py:45-60) over a ragged batch of camera-space clouds: the entry for scenes that do not come
+ * from a depth map (a reconstructed mesh, SLAM, a LiDAR sweep), whose grids reach the network as `scene_volumes=`.
+ * q_xy = ((p + s/2) * V) / s, q_z = (p_z * V) / s, round half-to-even, a point is kept iff 0 <= q <= V-1 on all three
+ * axes (-0.0 passes; NaN / inf points and overflowing products are dropped).  The precision follows the cloud's dtype,
+ * as in NumPy and torch: fp64 for f64 points, fp32 for f32 points; never contracted to FMA.
+ *   d_points    (total, 3) row-major, f64 (points_is_f64 = 1) or f32 (0)
+ *   d_offsets   (batch + 1) int64, device: frame b owns points [offsets[b], offsets[b+1]); non-decreasing, and
+ *               offsets[batch] <= total (the call cannot check this: the offsets live on the device)
+ *   d_occ_f32   (batch, V, V, V) f32, zeroed by the caller; occupied voxels set to 1.0
+ * batch == 0 launches nothing. */
+int sceneego_voxelize_points(const void* d_points, int points_is_f64, const int64_t* d_offsets, int batch,
+                             int volume_size, double cuboid_side, float* d_occ_f32, void* stream);
+
 /* with_intersection (network/voxel_net_depth.py:257-260): volumes = cat([volumes, volumes * scene, scene]).
  * In place on a plain planar bf16 volume whose channels [0,c) hold the lifted features and channel 2c the
  * occupancy: writes channels [c,2c) = features * occupancy at every voxel. */

@@ -48,7 +48,7 @@ SYMBOLS = [
     "sceneego_v2v_stem_s2d_weight_bytes", "sceneego_v2v_pack_stem_s2d", "sceneego_v2v_pack_conv_march", "sceneego_voxelize_depth_raw_f64", "sceneego_intersect_bf16", "sceneego_pose_errors_f64",
     "sceneego_voxelize_depth_dataset_f64", "sceneego_vol_layout_make_zwin", "sceneego_occ_expand_zwin_bf16", "sceneego_v2v_stem_march_weight_bytes",
     "sceneego_v2v_pack_stem_march", "sceneego_handoff_weight_bytes", "sceneego_handoff_workspace_bytes", "sceneego_handoff_pack",
-    "sceneego_backbone_handoff_f32",
+    "sceneego_backbone_handoff_f32", "sceneego_voxelize_points",
 ]
 
 
@@ -319,6 +319,36 @@ def voxelize_depth_dataset(depth_raw: torch.Tensor, pre_hw, clamp_max: float, ra
         raise SceneEgoError("voxelize_depth_dataset: the ray table must be (pre_h, pre_w, 3)")
     _call("sceneego_voxelize_depth_dataset_f64", depth_raw, depth_raw, b, h, w, int(pre_hw[0]), int(pre_hw[1]),
           C.c_float(clamp_max), ray, int(volume_size), C.c_double(cuboid_side), occ_f32)
+
+
+def voxelize_points(points: torch.Tensor, offsets: torch.Tensor, volume_size: int, cuboid_side: float,
+                    occ_f32: torch.Tensor) -> None:
+    """Ragged batch of camera-space clouds -> occupancy (point_cloud_to_voxel_numpy, network/voxel_net_depth.py:207-222):
+    points (N,3) float64 or float32 CUDA (computed in that precision), offsets (B+1,) int64 (frame b owns points
+    [offsets[b], offsets[b+1]); a CPU tensor is checked on the host and copied, a CUDA one is copied to the host to be
+    checked), occ_f32 (B,V,V,V) f32 zero-initialised; occupied voxels are set to 1."""
+    if not isinstance(points, torch.Tensor) or points.dtype not in (torch.float64, torch.float32):
+        raise SceneEgoError(f"voxelize_points: points must be a float64 or float32 tensor, got "
+                            f"{getattr(points, 'dtype', type(points).__name__)}")
+    if points.dim() != 2 or points.shape[1] != 3:
+        raise SceneEgoError(f"voxelize_points: points must have shape (N, 3), got {tuple(points.shape)}")
+    if not isinstance(offsets, torch.Tensor) or offsets.dtype != torch.int64 or offsets.dim() != 1 or offsets.numel() < 1:
+        raise SceneEgoError("voxelize_points: offsets must be a 1-D int64 tensor of B + 1 entries")
+    if not points.is_cuda:
+        raise SceneEgoError("voxelize_points: points must be a CUDA tensor (no CPU fallback)")
+    b, v = offsets.numel() - 1, int(volume_size)
+    if (not isinstance(occ_f32, torch.Tensor) or occ_f32.dtype != torch.float32 or tuple(occ_f32.shape) != (b, v, v, v)
+            or not occ_f32.is_cuda or occ_f32.device != points.device):
+        raise SceneEgoError(f"voxelize_points: occ_f32 must be a float32 ({b}, {v}, {v}, {v}) tensor on {points.device}")
+    o = offsets.cpu()
+    n = points.shape[0]
+    if int(o[0]) < 0 or int(o[-1]) > n or bool((o[1:] < o[:-1]).any()):
+        raise SceneEgoError(f"voxelize_points: offsets must be non-decreasing within [0, {n}]")
+    if b == 0 or int(o[-1]) == int(o[0]):
+        return                                       # nothing to scatter (an empty tensor may have no storage)
+    d_off = offsets if offsets.is_cuda and offsets.device == points.device else o.to(points.device)
+    _call("sceneego_voxelize_points", points, points, int(points.dtype == torch.float64), d_off.contiguous(), b, v,
+          C.c_double(cuboid_side), occ_f32)
 
 
 def occ_expand_zwin(occ_f32: torch.Tensor, vol: torch.Tensor, lay: VolLayout, channel: int) -> None:

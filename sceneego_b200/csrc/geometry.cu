@@ -393,8 +393,53 @@ __device__ __forceinline__ void set_occupied(__nv_bfloat16* __restrict__ occ, co
   }
 }
 
+// Round-to-nearest arithmetic of one precision, never contracted to FMA: the quantisation below is instantiated in
+// fp64 (depth maps; float64 clouds) and in fp32 (float32 clouds, which NumPy and torch keep in float32 when a Python
+// float is added or multiplied in).
+template <typename T> struct RnOps;
+template <> struct RnOps<double> {
+  static __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
+  static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
+  static __device__ __forceinline__ double div(double a, double b) { return __ddiv_rn(a, b); }
+  static __device__ __forceinline__ double round_even(double a) { return rint(a); }
+};
+template <> struct RnOps<float> {
+  static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
+  static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
+  static __device__ __forceinline__ float div(float a, float b) { return __fdiv_rn(a, b); }
+  static __device__ __forceinline__ float round_even(float a) { return rintf(a); }
+};
+
 // kPow2Side: 0 = divide by the cuboid side; 1 = the side is a power of two (x / 2^k == x * 2^-k exactly); 2 = the side AND
 // the volume size are powers of two: (x * V) * 2^-k == x * (V * 2^-k) exactly (both are exponent shifts), one multiply
+//
+// One camera-space point -> its voxel, point_cloud_to_voxel_numpy (network/voxel_net_depth.py:207-222) in the
+// reference's order: q_xy = ((p + s/2) * V) / s, q_z = (p_z * V) / s, round half-to-even, kept iff 0 <= q <= V-1 on all
+// three axes (-0.0 passes, as in NumPy; NaN / inf fail every comparison).  half = s/2, Vd = V, hi = V-1 in precision T.
+// voxelize_kernel keeps its own inline copy of the same fp64 steps: calling this helper from it changed that kernel's
+// SASS (its instruction count moved by up to 32 per instantiation in each form of the call tried).
+template <int kPow2Side, typename T>
+__device__ __forceinline__ bool quantize_point(T x, T y, T z, T half, T Vd, T side, T inv_side, T hi, int& ix, int& iy,
+                                               int& iz) {
+  using R = RnOps<T>;
+  const T mul = kPow2Side == 2 ? R::mul(Vd, inv_side) : Vd;     // exact: a power of two either way
+  T qx = R::mul(R::add(x, half), mul);
+  T qy = R::mul(R::add(y, half), mul);
+  T qz = R::mul(z, mul);
+  if (kPow2Side == 2) {
+  } else if (kPow2Side == 1) {   // x / 2^k == x * 2^-k exactly (no divide on the hot path)
+    qx = R::mul(qx, inv_side); qy = R::mul(qy, inv_side); qz = R::mul(qz, inv_side);
+  } else {
+    qx = R::div(qx, side); qy = R::div(qy, side); qz = R::div(qz, side);
+  }
+  qx = R::round_even(qx); qy = R::round_even(qy); qz = R::round_even(qz);
+  if (qx >= T(0) && qx <= hi && qy >= T(0) && qy <= hi && qz >= T(0) && qz <= hi) {
+    ix = (int)qx; iy = (int)qy; iz = (int)qz;
+    return true;
+  }
+  return false;
+}
+
 template <int kPow2Side>
 __global__ void __launch_bounds__(256) voxelize_kernel(const float* __restrict__ depth, int h, int w, NearestMaps nm,
                                                       const double* __restrict__ ray, int img_h, int img_w, int V,
@@ -484,6 +529,51 @@ __global__ void __launch_bounds__(256) voxelize_kernel(const float* __restrict__
       if (occ_f32) occ_f32[(((size_t)b * V + ix) * V + iy) * V + iz] = 1.0f;
       if (occ_bf16) set_occupied(occ_bf16, lay, b, ix, iy, iz, channel, V);
     }
+  }
+}
+
+// ---------------------------------------------------------------------------
+// point_cloud_to_voxel_numpy / point_cloud_to_voxel_pytorch over a ragged batch of camera-space clouds: frame b owns
+// points [offsets[b], offsets[b+1]).  One grid-stride loop over ALL points of the batch (the host does not know the
+// per-frame counts without a synchronisation, and a flat loop keeps every block busy however ragged the batch is); a
+// thread finds its frame by a binary search over `offsets` only when its point leaves the frame it was in.
+// Scatter: consecutive points of a cloud usually land in the same voxel (neighbouring pixels of a depth map, a wall,
+// the thousands of zero-depth points at (0,0,0)), so the lanes of a warp that target the same voxel elect one writer
+// (match.any): same-address stores serialise in L2, which is what voxelize_kernel's block vote on the zero-depth voxel
+// avoids as well.  Stores of 1.0 by different warps to one voxel are a benign race.
+// ---------------------------------------------------------------------------
+template <int kPow2Side, typename T>
+__global__ void __launch_bounds__(256) voxelize_points_kernel(const T* __restrict__ pts,
+                                                             const int64_t* __restrict__ offsets, int batch, int V,
+                                                             T half, T Vd, T side, T inv_side, T hi,
+                                                             float* __restrict__ occ) {
+  const int64_t begin = offsets[0], end = offsets[batch];
+  const int lane = threadIdx.x & 31;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;                 // a multiple of 32: warps stay whole
+  const int64_t vol = (int64_t)V * V * V;
+  int b = -1;
+  int64_t f_lo = 0, f_hi = -1;                                            // [f_lo, f_hi): points of frame b
+  for (int64_t base = begin + (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < end; base += stride) {
+    const int64_t i = base + lane;
+    long long key = -1;
+    if (i < end) {
+      if (i >= f_hi || i < f_lo) {
+        int lo = 0, hi_b = batch;                                          // last b with offsets[b] <= i
+        while (hi_b - lo > 1) {
+          const int mid = (lo + hi_b) >> 1;
+          if (__ldg(offsets + mid) <= i) lo = mid; else hi_b = mid;
+        }
+        b = lo;
+        f_lo = __ldg(offsets + b);
+        f_hi = __ldg(offsets + b + 1);
+      }
+      const T* p = pts + 3 * i;
+      int ix, iy, iz;
+      if (quantize_point<kPow2Side>(__ldcs(p), __ldcs(p + 1), __ldcs(p + 2), half, Vd, side, inv_side, hi, ix, iy, iz))
+        key = (long long)b * vol + ((int64_t)ix * V + iy) * V + iz;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, (unsigned long long)key);
+    if (key >= 0 && lane == __ffs(peers) - 1) occ[key] = 1.0f;
   }
 }
 
@@ -781,6 +871,47 @@ extern "C" int sceneego_voxelize_depth_dataset_f64(const float* d_depth_raw, int
   // dataset/real_depth_utils.py:29-43: the (pre_h, pre_w) map times the (pre_h, pre_w) ray table, pixel for pixel
   return voxelize_impl(d_depth_raw, batch, h, w, pre_h, pre_w, clamp_max, d_ray, pre_h, pre_w, V, side, d_occ_f32,
                        nullptr, nullptr, 0, stream, true);
+}
+
+template <typename T>
+static void launch_voxelize_points(const T* d_points, const int64_t* d_offsets, int batch, int V, double side,
+                                   float* d_occ, int blocks, cudaStream_t st) {
+  // fp32 clouds: NumPy / torch turn the Python float s/2 and the ints V, V-1 into float32 operands; s/2 is formed in
+  // fp64 first, like the reference's `s / 2`
+  const T half = (T)(side / 2), Vd = (T)V, s = (T)side, hi = (T)(V - 1);
+  int e2 = 0;
+  const bool pow2 = frexp(side, &e2) == 0.5;                    // side == 2^(e2-1): divide == exact multiply
+  const bool pow2_v = (V & (V - 1)) == 0;
+  const T inv = pow2 ? (T)(1.0 / side) : T(0);
+  if (pow2 && pow2_v)
+    voxelize_points_kernel<2, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, half, Vd, s, inv, hi, d_occ);
+  else if (pow2)
+    voxelize_points_kernel<1, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, half, Vd, s, inv, hi, d_occ);
+  else
+    voxelize_points_kernel<0, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, half, Vd, s, inv, hi, d_occ);
+}
+
+extern "C" int sceneego_voxelize_points(const void* d_points, int points_is_f64, const int64_t* d_offsets, int batch,
+                                        int volume_size, double cuboid_side, float* d_occ_f32, void* stream) {
+  SE_REQUIRE(volume_size > 0 && cuboid_side > 0 && batch >= 0, "voxelize_points: need volume_size > 0, cuboid_side > 0, batch >= 0");
+  SE_REQUIRE(volume_size <= 4096 && (double)batch * volume_size * volume_size * volume_size < 4.0e18,
+             "voxelize_points: occupancy grid too large");
+  SE_REQUIRE(d_points && d_offsets && d_occ_f32, "voxelize_points: null argument");
+  if (batch == 0) return SCENEEGO_OK;
+  int dev = 0, sms = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
+    set_error("voxelize_points: %s", cudaGetErrorString(cudaGetLastError()));
+    return SCENEEGO_E_CUDA;
+  }
+  const int blocks = 8 * sms;                                   // 2048 resident threads per SM, one wave
+  if (points_is_f64)
+    launch_voxelize_points((const double*)d_points, d_offsets, batch, volume_size, cuboid_side, d_occ_f32, blocks,
+                           (cudaStream_t)stream);
+  else
+    launch_voxelize_points((const float*)d_points, d_offsets, batch, volume_size, cuboid_side, d_occ_f32, blocks,
+                           (cudaStream_t)stream);
+  SE_CUDA_LAUNCH_CHECK("voxelize_points");
+  return SCENEEGO_OK;
 }
 
 extern "C" int sceneego_occ_expand_zwin_bf16(float* d_occ_f32, void* d_vol, const sceneego_vol_layout_t* lay, int batch,

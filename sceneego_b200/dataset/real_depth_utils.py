@@ -12,6 +12,10 @@ NOTE the dataset's `depth_map_to_voxel` is NOT the network's `depth_map_to_voxel
 the network's nearest squash to 1024x1024 and its 128 zero-padded columns (7,782 vs 8,331 occupied voxels on the
 demo frame img_001000).  Both are provided, each pinned against the reference function it replaces
 (tests/golden/voxel_dataset.npz, tests/golden/voxel.npz).
+
+Clouds that do not come from a depth map (a reconstructed mesh, SLAM, a LiDAR sweep) enter through
+`point_cloud_to_voxel_pytorch` (one cloud, :45-60) or `point_clouds_to_voxels` (a ragged batch, one launch of
+`sceneego_voxelize_points`); the grids go to the network as `scene_volumes=`.
 """
 from __future__ import annotations
 
@@ -76,6 +80,56 @@ def depth_maps_to_voxels(ray, depth_raw: torch.Tensor, cuboid_side: float, volum
     else:
         _lib.voxelize_depth_dataset(d, (PRE_H, PRE_W), clamp, r, volume_size, float(cuboid_side), occ)
     return occ
+
+
+def point_clouds_to_voxels(points, counts_or_offsets, cuboid_side: float, volume_size: int) -> torch.Tensor:
+    """Batch form of `point_cloud_to_voxel_pytorch` (one launch of `sceneego_voxelize_points`): a ragged batch of
+    camera-space clouds -> (B,V,V,V) f32 {0,1} on the clouds' device.
+
+    points: one (N,3) float64 / float32 CUDA tensor holding every frame's points back to back, or a list of (N_b,3)
+        tensors (concatenated on the device; they must share a dtype).  The arithmetic follows the dtype, like NumPy
+        and torch: float32 clouds are quantised in fp32, float64 clouds in fp64.
+    counts_or_offsets: B per-frame point counts, or B+1 offsets (frame b owns points [offsets[b], offsets[b+1])), as a
+        sequence, array or tensor.  Entries that sum to N are read as counts; otherwise they must be offsets (0 first,
+        N last, non-decreasing).  The two readings only collide for [0, ..., 0, N], which is read as counts.  None with
+        a list of clouds takes the list's lengths."""
+    if isinstance(points, (list, tuple)):
+        clouds = [torch.as_tensor(p) for p in points]
+        if not clouds:
+            raise _lib.SceneEgoError("point_clouds_to_voxels: empty list of clouds (pass a (0,3) tensor and counts)")
+        if any(c.dtype != clouds[0].dtype for c in clouds):
+            raise _lib.SceneEgoError("point_clouds_to_voxels: the clouds of a batch must share a dtype")
+        if counts_or_offsets is None:
+            counts_or_offsets = [c.reshape(-1, 3).shape[0] for c in clouds]
+        points = torch.cat([c.reshape(-1, 3) for c in clouds]) if len(clouds) > 1 else clouds[0]
+    if not isinstance(points, torch.Tensor) or not points.is_cuda:
+        raise _lib.SceneEgoError("point_clouds_to_voxels needs CUDA tensors (no CPU fallback)")
+    if counts_or_offsets is None:
+        raise _lib.SceneEgoError("point_clouds_to_voxels: per-frame counts or offsets are required with one tensor")
+    c = torch.as_tensor(counts_or_offsets).reshape(-1).to("cpu", torch.int64)
+    n = points.shape[0] if points.dim() == 2 else -1
+    if int(c.sum()) == n and not bool((c < 0).any()):
+        offsets = torch.cat([torch.zeros(1, dtype=torch.int64), torch.cumsum(c, 0)])
+    elif c.numel() >= 1 and int(c[0]) == 0 and int(c[-1]) == n and bool((c[1:] >= c[:-1]).all()):
+        offsets = c
+    else:
+        raise _lib.SceneEgoError(f"point_clouds_to_voxels: need B counts >= 0 summing to {n} points, or B+1 "
+                                 f"non-decreasing offsets from 0 to {n}")
+    v = int(volume_size)
+    occ = torch.zeros(offsets.numel() - 1, v, v, v, dtype=torch.float32, device=points.device)
+    _lib.voxelize_points(points.contiguous(), offsets, v, float(cuboid_side), occ)
+    return occ
+
+
+def point_cloud_to_voxel_pytorch(scene_point_cloud, cuboid_side, volume_size):
+    """dataset/real_depth_utils.py:45-60 for ONE camera-space cloud: (N,3) float64 / float32 tensor or array (CPU
+    inputs are copied to the current CUDA device) -> (V,V,V) f32 {0,1}.  Argument order (cloud, cuboid side, volume
+    size) as `depth_map_to_voxel` calls it (:29-43).  The quantisation runs in the cloud's precision."""
+    p = torch.as_tensor(scene_point_cloud)
+    if not p.is_cuda:
+        p = p.cuda()
+    p = p.reshape(-1, 3)
+    return point_clouds_to_voxels(p, [p.shape[0]], cuboid_side, volume_size)[0]
 
 
 def depth_map_to_voxel(ray, depth, cuboid_side, volume_size):

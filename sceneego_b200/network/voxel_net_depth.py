@@ -9,6 +9,7 @@ C-ABI of include/sceneego_b200.h:
                       unless `materialize_features`)      -> sceneego_feature_conv1x1_f32
     unproject_heatmaps_one_view_batch + torch.cat         -> sceneego_unproject_f32
     depth_map_to_voxel_numpy loop (host NumPy in the ref) -> sceneego_voxelize_depth_f64
+    point_cloud_to_voxel_numpy (clouds for scene_volumes=) -> sceneego_voxelize_points
     volume_net (V2VModel)                                 -> sceneego_v2v_run
     integrate_tensor_3d_with_coordinates                  -> sceneego_softargmax3d_f32
 
@@ -437,3 +438,24 @@ class VoxelNetwork_depth(nn.Module):
         _lib.voxelize_depth(d, self._ray_dev, self.image_height, self.image_width, self.volume_size,
                             float(self.cuboid_side), occ, None, None)
         return occ[0]
+
+    def point_cloud_to_voxel_numpy(self, scene_point_cloud):
+        """network/voxel_net_depth.py:207-222: one camera-space (N,3) cloud -- NumPy array or torch tensor, CPU (copied
+        to the module's device once) or CUDA -> (V,V,V) f32 {0,1} on the module's device, with the module's
+        `volume_size` and `cuboid_side`.  A float64 cloud is quantised in fp64 (what depth_map_to_voxel_numpy builds:
+        fp64 rays times depth), a float32 one in fp32, like NumPy.  Stack the grids of a batch and pass them as
+        `scene_volumes=`."""
+        p = torch.as_tensor(scene_point_cloud).reshape(-1, 3)
+        dev = _lib._as_device(self.device)
+        if p.device != dev:
+            p = p.to(dev)
+        occ = torch.zeros(1, self.volume_size, self.volume_size, self.volume_size, dtype=torch.float32, device=dev)
+        _lib.voxelize_points(p.contiguous(), torch.tensor([0, p.shape[0]], dtype=torch.int64), self.volume_size,
+                             float(self.cuboid_side), occ)
+        return occ[0]
+
+    def calculated_ray_direction_numpy(self, image_width, image_height):
+        """network/voxel_net_depth.py:147-155: the (W*H, 3) fp64 unit-ray table in the reference's x-major order
+        (row x*H + y), computed on the device (sceneego_ray_table_f64) and copied to the host as a NumPy array."""
+        ray = self.fisheye_camera_model.ray_table_device(image_width, image_height, _lib._as_device(self.device))
+        return ray.permute(1, 0, 2).reshape(-1, 3).cpu().numpy()
