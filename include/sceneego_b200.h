@@ -198,6 +198,19 @@ int sceneego_voxelize_depth_dataset_f64(const float* d_depth_raw, int batch, int
 int sceneego_voxelize_points(const void* d_points, int points_is_f64, const int64_t* d_offsets, int batch,
                              int volume_size, double cuboid_side, float* d_occ_f32, void* stream);
 
+/* The same occupancy for a static world-space scan seen from `batch` camera poses (a room from a mesh, SLAM or a LiDAR
+ * sweep, and the head-mounted camera's trajectory), in one launch and without a transformed copy of the scan.  Frame b's
+ * cloud is c_k = ((A[k,0]*x + A[k,1]*y) + A[k,2]*z) + t[k] for the (3,4) block [A|t] of its cam_from_world pose, each
+ * operation rounded in the points' precision (NumPy's `A[k,0]*x + A[k,1]*y + A[k,2]*z + t[k]`, no FMA); c is then
+ * quantised exactly as sceneego_voxelize_points does it.  The camera frame is the one ray x depth produces, in which the
+ * cuboid spans x, y in [-s/2, s/2], z in [0, s].  [A|t] is applied as given (no orthonormality check).
+ *   d_points          (n_points, 3) row-major world-space scan, f64 (points_is_f64 = 1) or f32 (0), shared by all frames
+ *   d_cam_from_world  (batch, 3, 4) row-major, the points' type: the upper rows of each 4x4 pose
+ *   d_occ_f32         (batch, V, V, V) f32, zeroed by the caller; occupied voxels set to 1.0
+ * batch == 0 or n_points == 0 launches nothing. */
+int sceneego_voxelize_scan(const void* d_points, int points_is_f64, int64_t n_points, const void* d_cam_from_world,
+                           int batch, int volume_size, double cuboid_side, float* d_occ_f32, void* stream);
+
 /* with_intersection (network/voxel_net_depth.py:257-260): volumes = cat([volumes, volumes * scene, scene]).
  * In place on a plain planar bf16 volume whose channels [0,c) hold the lifted features and channel 2c the
  * occupancy: writes channels [c,2c) = features * occupancy at every voxel. */

@@ -48,7 +48,7 @@ SYMBOLS = [
     "sceneego_v2v_stem_s2d_weight_bytes", "sceneego_v2v_pack_stem_s2d", "sceneego_v2v_pack_conv_march", "sceneego_voxelize_depth_raw_f64", "sceneego_intersect_bf16", "sceneego_pose_errors_f64",
     "sceneego_voxelize_depth_dataset_f64", "sceneego_vol_layout_make_zwin", "sceneego_occ_expand_zwin_bf16", "sceneego_v2v_stem_march_weight_bytes",
     "sceneego_v2v_pack_stem_march", "sceneego_handoff_weight_bytes", "sceneego_handoff_workspace_bytes", "sceneego_handoff_pack",
-    "sceneego_backbone_handoff_f32", "sceneego_voxelize_points",
+    "sceneego_backbone_handoff_f32", "sceneego_voxelize_points", "sceneego_voxelize_scan",
 ]
 
 
@@ -348,6 +348,44 @@ def voxelize_points(points: torch.Tensor, offsets: torch.Tensor, volume_size: in
         return                                       # nothing to scatter (an empty tensor may have no storage)
     d_off = offsets if offsets.is_cuda and offsets.device == points.device else o.to(points.device)
     _call("sceneego_voxelize_points", points, points, int(points.dtype == torch.float64), d_off.contiguous(), b, v,
+          C.c_double(cuboid_side), occ_f32)
+
+
+def voxelize_scan(scan: torch.Tensor, cam_from_world: torch.Tensor, volume_size: int, cuboid_side: float,
+                  occ_f32: torch.Tensor) -> None:
+    """One world-space scan seen from B camera poses -> B occupancy grids in one launch, without a transformed copy of
+    the scan: scan (N,3) float64 or float32 CUDA (computed in that precision), cam_from_world (B,4,4) of the scan's
+    dtype, CPU or CUDA (checked on the host: finite, bottom row exactly (0,0,0,1); the upper (3,4) block is applied as
+    given), occ_f32 (B,V,V,V) f32 zero-initialised; occupied voxels are set to 1."""
+    if not isinstance(scan, torch.Tensor) or scan.dtype not in (torch.float64, torch.float32):
+        raise SceneEgoError(f"voxelize_scan: scan must be a float64 or float32 tensor, got "
+                            f"{getattr(scan, 'dtype', type(scan).__name__)}")
+    if scan.dim() != 2 or scan.shape[1] != 3:
+        raise SceneEgoError(f"voxelize_scan: scan must have shape (N, 3), got {tuple(scan.shape)}")
+    if not isinstance(cam_from_world, torch.Tensor) or cam_from_world.dim() != 3 or tuple(cam_from_world.shape[1:]) != (4, 4):
+        raise SceneEgoError(f"voxelize_scan: cam_from_world must be a (B, 4, 4) tensor, got "
+                            f"{tuple(getattr(cam_from_world, 'shape', ())) or type(cam_from_world).__name__}")
+    if cam_from_world.dtype != scan.dtype:
+        raise SceneEgoError(f"voxelize_scan: cam_from_world must have the scan's dtype {scan.dtype}, got "
+                            f"{cam_from_world.dtype} (the transform runs in the scan's precision; cast explicitly)")
+    pose = cam_from_world.detach().cpu()
+    if not bool(torch.isfinite(pose).all()):
+        raise SceneEgoError("voxelize_scan: cam_from_world has non-finite entries")
+    bottom = torch.tensor([0.0, 0.0, 0.0, 1.0], dtype=pose.dtype)
+    if not bool((pose[:, 3, :] == bottom).all()):
+        raise SceneEgoError("voxelize_scan: the bottom row of every cam_from_world must be exactly (0, 0, 0, 1)")
+    b, v = pose.shape[0], int(volume_size)
+    if (not isinstance(occ_f32, torch.Tensor) or occ_f32.dtype != torch.float32
+            or tuple(occ_f32.shape) != (b, v, v, v)):
+        raise SceneEgoError(f"voxelize_scan: occ_f32 must be a float32 ({b}, {v}, {v}, {v}) tensor")
+    if not scan.is_cuda:
+        raise SceneEgoError("voxelize_scan: scan must be a CUDA tensor (no CPU fallback)")
+    if not occ_f32.is_cuda or occ_f32.device != scan.device:
+        raise SceneEgoError(f"voxelize_scan: occ_f32 must be on {scan.device}")
+    if b == 0 or scan.shape[0] == 0:
+        return                                       # nothing to scatter (an empty tensor may have no storage)
+    d_pose = pose[:, :3, :].contiguous().to(scan.device)
+    _call("sceneego_voxelize_scan", scan, scan, int(scan.dtype == torch.float64), C.c_int64(scan.shape[0]), d_pose, b, v,
           C.c_double(cuboid_side), occ_f32)
 
 

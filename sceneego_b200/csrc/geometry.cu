@@ -578,6 +578,59 @@ __global__ void __launch_bounds__(256) voxelize_points_kernel(const T* __restric
 }
 
 // ---------------------------------------------------------------------------
+// One world-space scan shared by `batch` frames, each with its own camera pose: frame b's cloud is
+// c_k = ((A[k,0]*x + A[k,1]*y) + A[k,2]*z) + t[k] for the (3,4) block [A|t] of cam_from_world[b] (NumPy's order for
+// `A[k,0]*x + A[k,1]*y + A[k,2]*z + t[k]`, every operation rounded, no FMA), then quantised by quantize_point like
+// voxelize_points_kernel.  The transformed clouds are never written: a thread loads a scan point once and evaluates it
+// for every frame of its block's frame tile (blockIdx.y), whose poses sit in shared memory.
+// kScanFrameTile = 32 frames per tile: the scan is read once per tile, i.e. 24 bytes (fp64) or 12 bytes (fp32) per point
+// against 32 transforms and quantisations.  The arithmetic dominates at that ratio (B = 64 on a B200 reads the scan at
+// 0.1-0.3 TB/s, DESIGN section 7), so a larger tile would save little traffic while leaving fewer (point block, frame
+// tile) pairs to spread a small scan over.
+// Scatter: per frame (uniform over the warp), lanes that hit the same voxel elect one writer, as in
+// voxelize_points_kernel: a dense scan puts many points into one voxel.
+// ---------------------------------------------------------------------------
+constexpr int kScanFrameTile = 32;
+
+template <int kPow2Side, typename T>
+__global__ void __launch_bounds__(256) voxelize_scan_kernel(const T* __restrict__ pts, int64_t n,
+                                                           const T* __restrict__ cam_from_world, int batch, int V,
+                                                           T half, T Vd, T side, T inv_side, T hi,
+                                                           float* __restrict__ occ) {
+  using R = RnOps<T>;
+  __shared__ T pose[kScanFrameTile][12];
+  const int b0 = blockIdx.y * kScanFrameTile;
+  const int nf = min(kScanFrameTile, batch - b0);
+  for (int e = threadIdx.x; e < nf * 12; e += blockDim.x) pose[e / 12][e % 12] = cam_from_world[(int64_t)b0 * 12 + e];
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;                 // a multiple of 32: warps stay whole
+  const int64_t vol = (int64_t)V * V * V;
+  for (int64_t base = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < n; base += stride) {
+    const int64_t i = base + lane;
+    T x = T(0), y = T(0), z = T(0);
+    if (i < n) {
+      const T* p = pts + 3 * i;
+      x = __ldg(p); y = __ldg(p + 1); z = __ldg(p + 2);
+    }
+    for (int f = 0; f < nf; ++f) {                                         // uniform over the block
+      const T* P = pose[f];
+      long long key = -1;
+      if (i < n) {
+        const T c0 = R::add(R::add(R::add(R::mul(P[0], x), R::mul(P[1], y)), R::mul(P[2], z)), P[3]);
+        const T c1 = R::add(R::add(R::add(R::mul(P[4], x), R::mul(P[5], y)), R::mul(P[6], z)), P[7]);
+        const T c2 = R::add(R::add(R::add(R::mul(P[8], x), R::mul(P[9], y)), R::mul(P[10], z)), P[11]);
+        int ix, iy, iz;
+        if (quantize_point<kPow2Side>(c0, c1, c2, half, Vd, side, inv_side, hi, ix, iy, iz))
+          key = (long long)(b0 + f) * vol + ((int64_t)ix * V + iy) * V + iz;
+      }
+      const unsigned peers = __match_any_sync(0xffffffffu, (unsigned long long)key);
+      if (key >= 0 && lane == __ffs(peers) - 1) occ[key] = 1.0f;
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------
 // z-window occupancy plane from a plain f32 occupancy grid (the marching stem's input, include/sceneego_b200.h):
 // cell (x,y,z) of plane channel/8 = occ[x][y][z-3 .. z+4] as eight 16-bit values.  voxelize_kernel can scatter into
 // that form directly (set_occupied: eight 2-byte stores and their bounds checks per occupied pixel), but the
@@ -873,22 +926,45 @@ extern "C" int sceneego_voxelize_depth_dataset_f64(const float* d_depth_raw, int
                        nullptr, nullptr, 0, stream, true);
 }
 
+// quantize_point's operands in the points' precision and which kPow2Side path applies
+template <typename T>
+struct PointQuant {
+  T half, Vd, s, inv, hi;
+  int path;
+  PointQuant(int V, double side) {
+    // fp32 clouds: NumPy / torch turn the Python float s/2 and the ints V, V-1 into float32 operands; s/2 is formed in
+    // fp64 first, like the reference's `s / 2`
+    half = (T)(side / 2); Vd = (T)V; s = (T)side; hi = (T)(V - 1);
+    int e2 = 0;
+    const bool pow2 = frexp(side, &e2) == 0.5;                  // side == 2^(e2-1): divide == exact multiply
+    const bool pow2_v = (V & (V - 1)) == 0;
+    inv = pow2 ? (T)(1.0 / side) : T(0);
+    path = pow2 && pow2_v ? 2 : pow2 ? 1 : 0;
+  }
+};
+
 template <typename T>
 static void launch_voxelize_points(const T* d_points, const int64_t* d_offsets, int batch, int V, double side,
                                    float* d_occ, int blocks, cudaStream_t st) {
-  // fp32 clouds: NumPy / torch turn the Python float s/2 and the ints V, V-1 into float32 operands; s/2 is formed in
-  // fp64 first, like the reference's `s / 2`
-  const T half = (T)(side / 2), Vd = (T)V, s = (T)side, hi = (T)(V - 1);
-  int e2 = 0;
-  const bool pow2 = frexp(side, &e2) == 0.5;                    // side == 2^(e2-1): divide == exact multiply
-  const bool pow2_v = (V & (V - 1)) == 0;
-  const T inv = pow2 ? (T)(1.0 / side) : T(0);
-  if (pow2 && pow2_v)
-    voxelize_points_kernel<2, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, half, Vd, s, inv, hi, d_occ);
-  else if (pow2)
-    voxelize_points_kernel<1, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, half, Vd, s, inv, hi, d_occ);
+  const PointQuant<T> q(V, side);
+  if (q.path == 2)
+    voxelize_points_kernel<2, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, q.half, q.Vd, q.s, q.inv, q.hi, d_occ);
+  else if (q.path == 1)
+    voxelize_points_kernel<1, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, q.half, q.Vd, q.s, q.inv, q.hi, d_occ);
   else
-    voxelize_points_kernel<0, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, half, Vd, s, inv, hi, d_occ);
+    voxelize_points_kernel<0, T><<<blocks, 256, 0, st>>>(d_points, d_offsets, batch, V, q.half, q.Vd, q.s, q.inv, q.hi, d_occ);
+}
+
+template <typename T>
+static void launch_voxelize_scan(const T* d_points, int64_t n, const T* d_pose, int batch, int V, double side,
+                                 float* d_occ, dim3 grid, cudaStream_t st) {
+  const PointQuant<T> q(V, side);
+  if (q.path == 2)
+    voxelize_scan_kernel<2, T><<<grid, 256, 0, st>>>(d_points, n, d_pose, batch, V, q.half, q.Vd, q.s, q.inv, q.hi, d_occ);
+  else if (q.path == 1)
+    voxelize_scan_kernel<1, T><<<grid, 256, 0, st>>>(d_points, n, d_pose, batch, V, q.half, q.Vd, q.s, q.inv, q.hi, d_occ);
+  else
+    voxelize_scan_kernel<0, T><<<grid, 256, 0, st>>>(d_points, n, d_pose, batch, V, q.half, q.Vd, q.s, q.inv, q.hi, d_occ);
 }
 
 extern "C" int sceneego_voxelize_points(const void* d_points, int points_is_f64, const int64_t* d_offsets, int batch,
@@ -911,6 +987,36 @@ extern "C" int sceneego_voxelize_points(const void* d_points, int points_is_f64,
     launch_voxelize_points((const float*)d_points, d_offsets, batch, volume_size, cuboid_side, d_occ_f32, blocks,
                            (cudaStream_t)stream);
   SE_CUDA_LAUNCH_CHECK("voxelize_points");
+  return SCENEEGO_OK;
+}
+
+extern "C" int sceneego_voxelize_scan(const void* d_points, int points_is_f64, int64_t n_points,
+                                      const void* d_cam_from_world, int batch, int volume_size, double cuboid_side,
+                                      float* d_occ_f32, void* stream) {
+  SE_REQUIRE(volume_size > 0 && cuboid_side > 0 && batch >= 0 && n_points >= 0,
+             "voxelize_scan: need volume_size > 0, cuboid_side > 0, batch >= 0, n_points >= 0");
+  SE_REQUIRE(volume_size <= 4096 && (double)batch * volume_size * volume_size * volume_size < 4.0e18,
+             "voxelize_scan: occupancy grid too large");
+  SE_REQUIRE(n_points <= INT64_MAX / 3 - 256, "voxelize_scan: too many points");
+  SE_REQUIRE(batch <= 65535LL * kScanFrameTile, "voxelize_scan: batch too large");
+  SE_REQUIRE(d_points && d_cam_from_world && d_occ_f32, "voxelize_scan: null argument");
+  if (batch == 0 || n_points == 0) return SCENEEGO_OK;
+  int dev = 0, sms = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
+    set_error("voxelize_scan: %s", cudaGetErrorString(cudaGetLastError()));
+    return SCENEEGO_E_CUDA;
+  }
+  // (point blocks, frame tiles): one resident wave of 2048 threads per SM over the point blocks of each tile, fewer
+  // when the scan is small; a block strides over the scan
+  const int64_t need = (n_points + 255) / 256;
+  const dim3 grid((unsigned)(need < 8LL * sms ? need : 8LL * sms), (unsigned)((batch + kScanFrameTile - 1) / kScanFrameTile));
+  if (points_is_f64)
+    launch_voxelize_scan((const double*)d_points, n_points, (const double*)d_cam_from_world, batch, volume_size,
+                         cuboid_side, d_occ_f32, grid, (cudaStream_t)stream);
+  else
+    launch_voxelize_scan((const float*)d_points, n_points, (const float*)d_cam_from_world, batch, volume_size,
+                         cuboid_side, d_occ_f32, grid, (cudaStream_t)stream);
+  SE_CUDA_LAUNCH_CHECK("voxelize_scan");
   return SCENEEGO_OK;
 }
 

@@ -15,7 +15,9 @@ demo frame img_001000).  Both are provided, each pinned against the reference fu
 
 Clouds that do not come from a depth map (a reconstructed mesh, SLAM, a LiDAR sweep) enter through
 `point_cloud_to_voxel_pytorch` (one cloud, :45-60) or `point_clouds_to_voxels` (a ragged batch, one launch of
-`sceneego_voxelize_points`); the grids go to the network as `scene_volumes=`.
+`sceneego_voxelize_points`); the grids go to the network as `scene_volumes=`.  A static world-space scan with one
+camera pose per frame enters through `scan_to_voxels` (one launch of `sceneego_voxelize_scan`, no per-frame copy of
+the scan).
 """
 from __future__ import annotations
 
@@ -118,6 +120,23 @@ def point_clouds_to_voxels(points, counts_or_offsets, cuboid_side: float, volume
     v = int(volume_size)
     occ = torch.zeros(offsets.numel() - 1, v, v, v, dtype=torch.float32, device=points.device)
     _lib.voxelize_points(points.contiguous(), offsets, v, float(cuboid_side), occ)
+    return occ
+
+
+def scan_to_voxels(scan, cam_from_world, cuboid_side: float, volume_size: int) -> torch.Tensor:
+    """One static world-space scan (a mesh, SLAM map or LiDAR sweep of the room) seen from B camera poses -> (B,V,V,V)
+    f32 {0,1}, one launch of `sceneego_voxelize_scan`; the per-frame transformed clouds are never materialised.
+
+    scan: (N,3) float64 / float32 CUDA tensor; the transform and the quantisation run in its precision.
+    cam_from_world: (B,4,4) poses of the scan's dtype (CPU or CUDA) mapping world points into the camera frame that
+        ray x depth produces; frame b's grid is `point_cloud_to_voxel_pytorch` of
+        `A[k,0]*x + A[k,1]*y + A[k,2]*z + t[k]` (that order, no FMA) with [A|t] = cam_from_world[b, :3]."""
+    if not isinstance(scan, torch.Tensor) or not scan.is_cuda:
+        raise _lib.SceneEgoError("scan_to_voxels needs a CUDA scan tensor (no CPU fallback)")
+    pose = torch.as_tensor(cam_from_world)
+    v = int(volume_size)
+    occ = torch.zeros(pose.shape[0] if pose.dim() == 3 else 0, v, v, v, dtype=torch.float32, device=scan.device)
+    _lib.voxelize_scan(scan.contiguous(), pose, v, float(cuboid_side), occ)
     return occ
 
 

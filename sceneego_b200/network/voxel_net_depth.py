@@ -10,6 +10,7 @@ C-ABI of include/sceneego_b200.h:
     unproject_heatmaps_one_view_batch + torch.cat         -> sceneego_unproject_f32
     depth_map_to_voxel_numpy loop (host NumPy in the ref) -> sceneego_voxelize_depth_f64
     point_cloud_to_voxel_numpy (clouds for scene_volumes=) -> sceneego_voxelize_points
+    scan_to_voxels (world scan + B poses, scene_volumes=)   -> sceneego_voxelize_scan
     volume_net (V2VModel)                                 -> sceneego_v2v_run
     integrate_tensor_3d_with_coordinates                  -> sceneego_softargmax3d_f32
 
@@ -453,6 +454,23 @@ class VoxelNetwork_depth(nn.Module):
         _lib.voxelize_points(p.contiguous(), torch.tensor([0, p.shape[0]], dtype=torch.int64), self.volume_size,
                              float(self.cuboid_side), occ)
         return occ[0]
+
+    def scan_to_voxels(self, scan, cam_from_world):
+        """One static world-space (N,3) scan and B (4,4) cam_from_world poses -- NumPy arrays or torch tensors, CPU
+        (the scan is copied to the module's device) or CUDA -> (B,V,V,V) f32 {0,1} on the module's device, with the
+        module's `volume_size` and `cuboid_side`, in one launch (sceneego_voxelize_scan).  Frame b's grid is
+        point_cloud_to_voxel_numpy of the scan mapped into camera b's frame (the frame of ray x depth) by
+        `A[k,0]*x + A[k,1]*y + A[k,2]*z + t[k]` in the scan's precision; the poses must have the scan's dtype.
+        Pass the result as `scene_volumes=`."""
+        p = torch.as_tensor(scan)
+        dev = _lib._as_device(self.device)
+        if p.device != dev:
+            p = p.to(dev)
+        v = self.volume_size
+        pose = torch.as_tensor(cam_from_world)
+        occ = torch.zeros(pose.shape[0] if pose.dim() == 3 else 0, v, v, v, dtype=torch.float32, device=dev)
+        _lib.voxelize_scan(p.contiguous(), pose, v, float(self.cuboid_side), occ)
+        return occ
 
     def calculated_ray_direction_numpy(self, image_width, image_height):
         """network/voxel_net_depth.py:147-155: the (W*H, 3) fp64 unit-ray table in the reference's x-major order

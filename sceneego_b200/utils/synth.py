@@ -93,6 +93,62 @@ def synthetic_depth_room(batch: int, ray: np.ndarray, seed: int = 7, h: int = 10
     return torch.from_numpy(out)
 
 
+ROOM_SIZE = (10.0, 8.0, 3.0)      # synthetic_world_scan's room: x, y extent of the floor and the height, metres
+
+
+def synthetic_world_scan(n: int, seed: int = 0, dtype=np.float64) -> np.ndarray:
+    """A static world-space scan like a mesh, SLAM map or LiDAR sweep would give: n points sampled uniformly by area
+    from the floor (z = 0), the four walls and the ceiling of a ROOM_SIZE room, and the five visible faces of four
+    boxes standing on the floor, with 5 mm of noise.  World z points up.  (n,3) in `dtype`."""
+    rng = np.random.default_rng(seed)
+    W, D, H = ROOM_SIZE
+    # axis-aligned rectangles: (origin, edge u, edge v)
+    rects = [((0, 0, 0), (W, 0, 0), (0, D, 0)), ((0, 0, H), (W, 0, 0), (0, D, 0)),
+             ((0, 0, 0), (W, 0, 0), (0, 0, H)), ((0, D, 0), (W, 0, 0), (0, 0, H)),
+             ((0, 0, 0), (0, D, 0), (0, 0, H)), ((W, 0, 0), (0, D, 0), (0, 0, H))]
+    for _ in range(4):
+        sx, sy, sz = rng.uniform(0.4, 1.2), rng.uniform(0.4, 1.2), rng.uniform(0.3, 1.0)
+        ox, oy = rng.uniform(0.5, W - 0.5 - sx), rng.uniform(0.5, D - 0.5 - sy)
+        rects += [((ox, oy, sz), (sx, 0, 0), (0, sy, 0)),
+                  ((ox, oy, 0), (sx, 0, 0), (0, 0, sz)), ((ox, oy + sy, 0), (sx, 0, 0), (0, 0, sz)),
+                  ((ox, oy, 0), (0, sy, 0), (0, 0, sz)), ((ox + sx, oy, 0), (0, sy, 0), (0, 0, sz))]
+    o, u, v = (np.array([r[i] for r in rects], np.float64) for i in range(3))
+    area = np.linalg.norm(np.cross(u, v), axis=1)
+    k = rng.choice(len(rects), size=n, p=area / area.sum())
+    a, b = rng.random((n, 1)), rng.random((n, 1))
+    pts = o[k] + a * u[k] + b * v[k] + rng.normal(0.0, 0.005, (n, 3))
+    return pts.astype(dtype)
+
+
+def synthetic_head_trajectory(batch: int, seed: int = 0, dtype=np.float64) -> np.ndarray:
+    """(batch,4,4) cam_from_world poses of a head-mounted, downward-looking fisheye camera walking a smooth loop in
+    synthetic_world_scan's room: head height 1.5-1.8 m, optical axis (camera z) tilted up to ~0.35 rad from straight
+    down, heading turning through the walk.  The head stays at least 3 m from every wall, so the network's cuboid
+    (x, y in [-s/2, s/2], z in [0, s] in the camera frame) stays within the walls for s <= 2.5; its far face passes
+    below the floor, as it does for a standing person.  Rigid: cam_from_world = [R^T | -R^T c] for the camera's
+    world orientation R and centre c, computed in fp64 and rounded to `dtype`."""
+    rng = np.random.default_rng(seed)
+    W, D, _ = ROOM_SIZE
+    t = np.arange(batch, dtype=np.float64) / max(batch, 1)
+    ph = rng.uniform(0, 2 * np.pi, 5)
+    cx = W / 2 + 1.5 * np.sin(2 * np.pi * t + ph[0])
+    cy = D / 2 + 0.8 * np.sin(4 * np.pi * t + ph[1])
+    cz = 1.65 + 0.15 * np.sin(6 * np.pi * t + ph[2])
+    yaw = ph[3] + 2 * np.pi * t
+    tilt = 0.2 + 0.15 * np.sin(2 * np.pi * 3 * t + ph[4])
+    out = np.zeros((batch, 4, 4), np.float64)
+    for i in range(batch):
+        zc = np.array([np.sin(tilt[i]) * np.cos(yaw[i]), np.sin(tilt[i]) * np.sin(yaw[i]), -np.cos(tilt[i])])
+        xc = np.array([-np.sin(yaw[i]), np.cos(yaw[i]), 0.0])
+        yc = np.cross(zc, xc)
+        R = np.stack([xc, yc, zc], axis=1)                  # columns: camera axes in world coordinates
+        c = np.array([cx[i], cy[i], cz[i]])
+        out[i, :3, :3] = R.T
+        out[i, :3, 3] = -R.T @ c
+        out[i, 3, 3] = 1.0
+    return out.astype(dtype)
+
+
 def stage_state_shapes(with_intersection: bool = False, num_joints: int = 15):
     """(key, shape) of every post-backbone state-dict entry of VoxelNetwork_depth (`process_features.*`,
     `volume_net.*`), derived from the module classes themselves (no GPU, no golden manifest needed)."""
