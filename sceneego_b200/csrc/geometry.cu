@@ -115,7 +115,9 @@ __global__ void __launch_bounds__(256) grid_sample_kernel(const float* __restric
   const float iy = __fmul_rn(__fdiv_rn(__fadd_rn(g.y, 1.0f), 2.0f), (float)(H - 1));
   const float x0f = floorf(ix), y0f = floorf(iy);
   const float wx1 = ix - x0f, wy1 = iy - y0f, wx0 = (x0f + 1.0f) - ix, wy0 = (y0f + 1.0f) - iy;
-  const int x0 = (int)x0f, y0 = (int)y0f;
+  // clamped before the conversion: far outside (|g| ~ 1e30) (int) saturates at INT_MAX and x0 + 1 would overflow,
+  // which the compiler may fold into a bounds test that passes; a clamped corner keeps both taps outside
+  const int x0 = (int)fminf(fmaxf(x0f, -2.0f), (float)W), y0 = (int)fminf(fmaxf(y0f, -2.0f), (float)H);
   float wt[4];
   int off[4];
 #pragma unroll
@@ -276,7 +278,7 @@ __global__ void __launch_bounds__(128) unproject_kernel(const float* __restrict_
   const float x0f = floorf(ix), y0f = floorf(iy);
   const float wx1 = ix - x0f, wy1 = iy - y0f;
   const float wx0 = (x0f + 1.0f) - ix, wy0 = (y0f + 1.0f) - iy;
-  const int x0 = (int)x0f, y0 = (int)y0f;
+  const int x0 = (int)fminf(fmaxf(x0f, -2.0f), (float)img_w), y0 = (int)fminf(fmaxf(y0f, -2.0f), (float)img_h);   // as in grid_sample_kernel
   const int pad = (img_w - img_h) / 2;
 
   // The image plane is the 16x nearest-upsampled source, so the four bilinear taps usually (88 % of the

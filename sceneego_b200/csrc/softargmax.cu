@@ -59,6 +59,8 @@ __global__ void __launch_bounds__(SA_THREADS) softargmax_partial_kernel(
         a.s *= f; a.sx *= f; a.sy *= f; a.sz *= f;
         a.m = mx;
       }
+      // every logit this thread has seen is -inf: their weights are 0, but exp2f(-inf - -inf) would make them NaN
+      if (a.m == -INFINITY) continue;
     }
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
