@@ -4,8 +4,8 @@
 //   umeyama           utils/rigid_transform_with_scale.py:18-43   c, R, t minimising sum |P c R + t - Q|^2
 // One thread = one frame, fp64 throughout (the reference runs NumPy float64: ground truth is stored in double).
 // The 3x3 SVD of the cross-covariance C = V S W is obtained from the symmetric eigenproblem C^T C = W^T S^2 W
-// (cyclic Jacobi, converges to machine precision in a few sweeps), V = C W^T S^-1, the last column completed by a
-// cross product when the third singular value vanishes (planar / collinear poses).
+// (cyclic Jacobi, converges to machine precision in a few sweeps); V's first two columns come from C W^T, its third is
+// their cross product, so V is orthonormal for planar and collinear poses too.
 #include "common.cuh"
 #include <math.h>
 
@@ -108,21 +108,37 @@ __global__ void __launch_bounds__(128) pose_errors_kernel(const TP* __restrict__
   Mat3 CtC, W, V;
   for (int i = 0; i < 3; ++i)
     for (int k = 0; k < 3; ++k) CtC.m[i][k] = C.m[0][i] * C.m[0][k] + C.m[1][i] * C.m[1][k] + C.m[2][i] * C.m[2][k];
-  double ev[3], S[3];
+  double ev[3], S[3], U[3][3];
   jacobi_eig3(CtC, ev, W);
   for (int i = 0; i < 3; ++i) S[i] = sqrt(ev[i] > 0.0 ? ev[i] : 0.0);
   const double tiny = 1e-14 * (S[0] > 0.0 ? S[0] : 1.0);
-  for (int c = 0; c < 3; ++c) {                                // V[:, c] = C W[c, :]^T / S[c]
-    if (S[c] > tiny) {
-      for (int i = 0; i < 3; ++i) V.m[i][c] = (C.m[i][0] * W.m[c][0] + C.m[i][1] * W.m[c][1] + C.m[i][2] * W.m[c][2]) / S[c];
-    } else if (c == 2) {                                       // rank 2: complete the basis
-      V.m[0][2] = V.m[1][0] * V.m[2][1] - V.m[2][0] * V.m[1][1];
-      V.m[1][2] = V.m[2][0] * V.m[0][1] - V.m[0][0] * V.m[2][1];
-      V.m[2][2] = V.m[0][0] * V.m[1][1] - V.m[1][0] * V.m[0][1];
-    } else {
-      for (int i = 0; i < 3; ++i) V.m[i][c] = i == c ? 1.0 : 0.0;   // rank <= 1: degenerate pose, any frame
+  for (int c = 0; c < 3; ++c)                                  // U[c] = C W[c, :]^T = S[c] V[:, c]
+    for (int i = 0; i < 3; ++i) U[c][i] = C.m[i][0] * W.m[c][0] + C.m[i][1] * W.m[c][1] + C.m[i][2] * W.m[c][2];
+  // V is made orthonormal from its first two columns.  A singular value below ~1e-8 S[0] is eigenvalue noise of
+  // C^T C (absolute error ~eps S[0]^2), so U[c] / S[c] is not a unit vector there: near-planar poses would get a
+  // non-orthogonal R.  Column 1 is U[1] orthogonalised against column 0 and normalised, or any unit vector orthogonal
+  // to it (rank <= 1: the rotation is not unique); column 2 is col0 x col1, so R = V W needs no third singular vector.
+  for (int i = 0; i < 3; ++i)
+    for (int k = 0; k < 3; ++k) V.m[i][k] = i == k ? 1.0 : 0.0;   // rank 0: V = I
+  const double n0 = sqrt(U[0][0] * U[0][0] + U[0][1] * U[0][1] + U[0][2] * U[0][2]);
+  if (S[0] > tiny && n0 > 0.0) {
+    double v0[3], v1[3];
+    for (int i = 0; i < 3; ++i) v0[i] = U[0][i] / n0;
+    const double p = v0[0] * U[1][0] + v0[1] * U[1][1] + v0[2] * U[1][2];
+    for (int i = 0; i < 3; ++i) v1[i] = U[1][i] - p * v0[i];
+    double n1 = sqrt(v1[0] * v1[0] + v1[1] * v1[1] + v1[2] * v1[2]);
+    if (!(S[1] > tiny && n1 > tiny)) {                         // rank 1: v0 x (the axis least aligned with v0)
+      const int k = fabs(v0[0]) <= fabs(v0[1]) ? (fabs(v0[0]) <= fabs(v0[2]) ? 0 : 2) : (fabs(v0[1]) <= fabs(v0[2]) ? 1 : 2);
+      const int k1 = (k + 1) % 3, k2 = (k + 2) % 3;
+      v1[k] = 0.0; v1[k1] = v0[k2]; v1[k2] = -v0[k1];          // v0 x e_k
+      n1 = sqrt(v1[k1] * v1[k1] + v1[k2] * v1[k2]);
     }
+    for (int i = 0; i < 3; ++i) { V.m[i][0] = v0[i]; V.m[i][1] = v1[i] / n1; }
+    V.m[0][2] = V.m[1][0] * V.m[2][1] - V.m[2][0] * V.m[1][1];
+    V.m[1][2] = V.m[2][0] * V.m[0][1] - V.m[0][0] * V.m[2][1];
+    V.m[2][2] = V.m[0][0] * V.m[1][1] - V.m[1][0] * V.m[0][1];
   }
+  for (int c = 0; c < 3; ++c) S[c] = V.m[0][c] * U[c][0] + V.m[1][c] * U[c][1] + V.m[2][c] * U[c][2];   // trace terms
   if (det3(V) * det3(W) < 0.0) {
     S[2] = -S[2];
     for (int i = 0; i < 3; ++i) V.m[i][2] = -V.m[i][2];

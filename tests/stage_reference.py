@@ -309,3 +309,131 @@ def assert_equal_flat(got, want, where, limit=8):
             t = tuple(row)
             lines.append(f"  {t}: got {g[t].item()!r}, want {w[t].item()!r}")
         raise AssertionError("\n".join(lines))
+
+
+# ---- fisheye projection (csrc/geometry.cu project_voxel) ----------------------------------------------------------------
+ATANF_ULP = 2         # atanf: 2 ulp over the full range (CUDA 12.9 Math API, single-precision functions table)
+TAU32 = 2.0 ** -150   # absolute rounding error of an fp32 result in the subnormal range
+
+
+def _ulp32(x):
+    """ulp of an fp32 value of magnitude <= |x| + ... (normal range; 2^-149 below it)."""
+    e = np.floor(np.log2(np.maximum(np.abs(x), 2.0 ** -126)))
+    return np.exp2(e - 23)
+
+
+def w2c_coeffs(calib):
+    """The kernel's fp32 copies of the W2C polynomial and the centre, as float64 values."""
+    a = np.asarray(calib["w2c"], np.float64).astype(np.float32).astype(np.float64)
+    cx, cy = (np.float64(np.float32(v)) for v in calib["center"])
+    return a, cx, cy
+
+
+def project_ref(pts, calib):
+    """Float64 value of the Scaramuzza expression at fp32 points (N, 3), with a running error bound of the fp32
+    evaluation (u = 2^-24 per rounded op plus 2^-150 absolute for subnormal results, sqrtf correctly rounded, atanf
+    ATANF_ULP ulp; input errors propagated through each op's derivative).  Returns (px (N, 2), radius (N, 2), theta,
+    r2_32), r2_32 being the fp32 value of X^2 + Y^2 (0 where the kernel takes its r == 0 branch)."""
+    a, cx, cy = w2c_coeffs(calib)
+    p = np.asarray(pts, np.float32).astype(np.float64)
+    X, Y, z = p[:, 0], p[:, 1], -p[:, 2]
+    rnd = lambda v, e: U32 * (np.abs(v) + e) + TAU32         # rounding of a result v known to within e
+    X2, Y2 = X * X, Y * Y
+    eX2, eY2 = rnd(X2, 0), rnd(Y2, 0)
+    s = X2 + Y2
+    es = eX2 + eY2
+    es = es + rnd(s, es)
+    r = np.sqrt(s)
+    er = es / (r + np.sqrt(np.maximum(s - es, 0.0)))
+    er = er + rnd(r, er)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        lo = np.maximum(r - er, 0.0)
+        q = z / r
+        eq = np.abs(z) * er / (r * lo)
+        eq = eq + rnd(q, eq)
+        th = np.arctan(q)
+        qlo = np.maximum(np.abs(q) - eq, 0.0)
+        eth = eq / (1.0 + qlo * qlo)
+        eth = eth + ATANF_ULP * _ulp32(np.abs(th) + eth)
+        inv = 1.0 / r
+        einv = er / (r * lo)
+        einv = einv + rnd(inv, einv)
+        t, et = np.ones_like(th), np.zeros_like(th)
+        rho, erho = np.full_like(th, a[0]), np.zeros_like(th)
+        for i in range(1, 11):
+            tn = t * th
+            etn = np.abs(t) * eth + np.abs(th) * et + et * eth
+            t, et = tn, etn + rnd(tn, etn)
+            m = t * a[i]
+            em = abs(a[i]) * et
+            em = em + rnd(m, em)
+            rho = rho + m
+            erho = erho + em
+            erho = erho + rnd(rho, erho)
+        out, rad = [], []
+        for V, c0 in ((X, cx), (Y, cy)):
+            xi = V * inv
+            exi = np.abs(V) * einv
+            exi = exi + rnd(xi, exi)
+            pm = xi * rho
+            epm = np.abs(xi) * erho + np.abs(rho) * exi + exi * erho
+            epm = epm + rnd(pm, epm)
+            px = pm + c0
+            epx = epm + rnd(px, epm)
+            out.append(px)
+            rad.append(1.001 * epx + 2.0 ** -40 * np.abs(px))   # the float64 evaluation itself
+    x32, y32 = p[:, 0].astype(np.float32), p[:, 1].astype(np.float32)
+    with np.errstate(over="ignore", under="ignore"):
+        r2_32 = (x32 * x32 + y32 * y32).astype(np.float64)
+    return np.stack(out, 1), np.stack(rad, 1), th, r2_32
+
+
+def normalise_ref(px, rad, hm_h, hm_w):
+    """g = 2 (p / [W, H] - 0.5) in fp32 (division, subtraction, exact doubling) around the projection's bound."""
+    out, orad = [], []
+    for k, size in ((0, hm_w), (1, hm_h)):
+        d = px[:, k] / size
+        ed = rad[:, k] / size
+        ed = ed + U32 * (np.abs(d) + ed) + TAU32
+        s = d - 0.5
+        es = ed + U32 * (np.abs(s) + ed) + TAU32
+        out.append(2 * s)
+        orad.append(2 * es)
+    return np.stack(out, 1), np.stack(orad, 1)
+
+
+def simulate_project_f32(pts, calib, atan_ulps=0, seed=0, drop=None, swap_centre=False, no_flip=False):
+    """The kernel in NumPy float32: atan perturbed by up to `atan_ulps` ulp (random direction per point); planted
+    defects: drop=i leaves out coefficient a_i, swap_centre exchanges cx and cy, no_flip takes theta from +Z."""
+    a, cx, cy = w2c_coeffs(calib)
+    a = a.astype(np.float32)
+    if swap_centre:
+        cx, cy = cy, cx
+    cx, cy = np.float32(cx), np.float32(cy)
+    p = np.asarray(pts, np.float32)
+    X, Y = p[:, 0], p[:, 1]
+    z = p[:, 2] if no_flip else p[:, 2] * np.float32(-1)
+    with np.errstate(all="ignore"):
+        r = np.sqrt(X * X + Y * Y)
+        th = np.arctan(z / r).astype(np.float32)
+        if atan_ulps:
+            rng = np.random.default_rng(seed)
+            k = rng.integers(-atan_ulps, atan_ulps + 1, th.shape)
+            for _ in range(atan_ulps):
+                th = np.where(k > 0, np.nextafter(th, np.float32(np.inf)), np.where(k < 0, np.nextafter(th, np.float32(-np.inf)), th))
+                k = k - np.sign(k)
+        inv = np.float32(1) / r
+        rho = np.full_like(th, a[0])
+        t = np.ones_like(th)
+        for i in range(1, 11):
+            t = t * th
+            if i != drop:
+                rho = rho + t * a[i]
+        px = (X * inv) * rho + cx
+        py = (Y * inv) * rho + cy
+    return np.stack([px, py], 1).astype(np.float64)
+
+
+def w2c_within(got, ref, rad):
+    got = np.asarray(got, np.float64)
+    return np.isfinite(got) & (np.abs(got - ref) <= rad)
