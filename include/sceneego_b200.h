@@ -27,6 +27,8 @@ extern "C" {
 #endif
 
 #define SCENEEGO_ABI_VERSION 5
+/* Most cameras one call of sceneego_unproject_cameras_f32 / sceneego_voxelize_depth_cameras_f64 takes. */
+#define SCENEEGO_MAX_CAMERAS 16
 
 enum {
   SCENEEGO_OK = 0,
@@ -139,6 +141,23 @@ int sceneego_unproject_f32(const float* d_feat, const float* d_grid, const scene
                            int img_h, int img_w, float* d_out_f32, void* d_out_bf16,
                            const sceneego_vol_layout_t* lay, int extra_zero_planes, void* stream);
 
+/* Same gather with a camera per frame, for batches that mix recordings from several fisheye lenses: frame b is
+ * sampled exactly as sceneego_unproject_f32 samples it with camera d_frame_camera[b] (bit for bit).
+ *   d_grids  (K,N,2) f32 stacked table-mode grids, row k for camera k; or NULL for fused mode, where
+ *   calibs   (host array of K) gives camera k's coefficients
+ *   n_cameras K in [1, SCENEEGO_MAX_CAMERAS]
+ *   d_frame_camera (B) int32, device: camera of frame b; every entry must lie in [0, K) (the call cannot check this:
+ *            the ids live on the device)
+ *   d_frame_order  (B) int32, device, or NULL = identity: a permutation of [0, B) in which frames are visited; with
+ *            frames that share a camera adjacent (a stable sort by camera), a voxel's geometry is computed once per
+ *            run of equal cameras instead of once per frame.  Outputs go to frame b's own slot whatever the order.
+ * The other arguments are those of sceneego_unproject_f32. */
+int sceneego_unproject_cameras_f32(const float* d_feat, const float* d_grids, const sceneego_calib_t* calibs,
+                                   int n_cameras, const int32_t* d_frame_camera, const int32_t* d_frame_order,
+                                   int batch, int h, int w, int c, int volume_size, float cuboid_side, int img_h,
+                                   int img_w, float* d_out_f32, void* d_out_bf16, const sceneego_vol_layout_t* lay,
+                                   int extra_zero_planes, void* stream);
+
 /* Generic bilinear gather with the reference op's own signature: replaces
  * F.grid_sample(heatmaps, grid, align_corners=True) at utils/op.py:209 (and :163) on a
  * materialised image.  d_img (B,C,H,W) f32 NCHW; d_grid (N,2) normalised coords, frame b
@@ -173,6 +192,19 @@ int sceneego_voxelize_depth_raw_f64(const float* d_depth_raw, int batch, int h, 
                                     float clamp_max, const double* d_ray, int img_h, int img_w, int volume_size,
                                     double cuboid_side, float* d_occ_f32, void* d_occ_bf16,
                                     const sceneego_vol_layout_t* lay, int channel, void* stream);
+
+/* sceneego_voxelize_depth_raw_f64 with a camera per frame: frame b back-projects through ray table d_frame_camera[b]
+ * and its occupancy equals, bit for bit, that call's with that camera's table.  pre_h == h, pre_w == w and
+ * clamp_max = +inf give sceneego_voxelize_depth_f64.
+ *   d_rays   (K, img_h, img_w, 3) fp64, K tables from sceneego_ray_table_f64 stacked;  n_cameras K in [1, SCENEEGO_MAX_CAMERAS]
+ *   d_frame_camera (B) int32, device, entries in [0, K) (not checked: they live on the device)
+ *   d_frame_order  (B) int32, device, or NULL = identity: a permutation of [0, B); a block's frames are taken in this
+ *            order and a pixel's ray is reloaded only when the camera changes (pass a stable sort by camera) */
+int sceneego_voxelize_depth_cameras_f64(const float* d_depth, int batch, int h, int w, int pre_h, int pre_w,
+                                        float clamp_max, const double* d_rays, int n_cameras,
+                                        const int32_t* d_frame_camera, const int32_t* d_frame_order, int img_h,
+                                        int img_w, int volume_size, double cuboid_side, float* d_occ_f32,
+                                        void* d_occ_bf16, const sceneego_vol_layout_t* lay, int channel, void* stream);
 
 /* The DATASET's voxelisation -- replaces depth_map_to_voxel / point_cloud_to_voxel_pytorch
  * (dataset/real_depth_utils.py:29-60), the voxel_output=True path of dataset/demo_dataset.py:93-94 and

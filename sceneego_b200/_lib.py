@@ -49,7 +49,9 @@ SYMBOLS = [
     "sceneego_voxelize_depth_dataset_f64", "sceneego_vol_layout_make_zwin", "sceneego_occ_expand_zwin_bf16", "sceneego_v2v_stem_march_weight_bytes",
     "sceneego_v2v_pack_stem_march", "sceneego_handoff_weight_bytes", "sceneego_handoff_workspace_bytes", "sceneego_handoff_pack",
     "sceneego_backbone_handoff_f32", "sceneego_voxelize_points", "sceneego_voxelize_scan",
+    "sceneego_unproject_cameras_f32", "sceneego_voxelize_depth_cameras_f64",
 ]
+MAX_CAMERAS = 16          # SCENEEGO_MAX_CAMERAS
 
 
 class Calib(C.Structure):
@@ -290,6 +292,48 @@ def unproject(feat_cl: torch.Tensor, grid: Optional[torch.Tensor], calib: Option
     _call("sceneego_unproject_f32", feat_cl, feat_cl, grid, C.byref(calib) if calib is not None else None, b, h, w, c,
           int(volume_size), C.c_float(cuboid_side), int(img_h), int(img_w), out_f32, out_bf16,
           C.byref(lay) if lay is not None else None, int(extra_zero_planes))
+
+
+def _frame_ids(t: Optional[torch.Tensor], b: int, what: str) -> None:
+    if t is not None and (not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or tuple(t.shape) != (b,)):
+        raise SceneEgoError(f"{what} must be a ({b},) int32 tensor")
+
+
+def unproject_cameras(feat_cl: torch.Tensor, grids: Optional[torch.Tensor], calibs, frame_camera: torch.Tensor,
+                      frame_order: Optional[torch.Tensor], volume_size: int, cuboid_side: float, img_h: int, img_w: int,
+                      out_f32: Optional[torch.Tensor], out_bf16: Optional[torch.Tensor], lay: Optional[VolLayout],
+                      extra_zero_planes: int = 0) -> None:
+    """`unproject` with a camera per frame: grids (K,N,2) f32 stacked tables (table mode) or None with `calibs`, a
+    sequence of K Calib (fused mode); frame_camera (B,) int32 CUDA with entries in [0, K); frame_order (B,) int32 CUDA
+    permutation (a stable sort by camera) or None."""
+    b, h, w, c = feat_cl.shape
+    n = int(volume_size) ** 3
+    if grids is not None and (grids.dim() != 3 or tuple(grids.shape[1:]) != (n, 2) or grids.dtype != torch.float32):
+        raise SceneEgoError(f"unproject_cameras: grids must be a (K, {n}, 2) float32 tensor")
+    k = grids.shape[0] if grids is not None else len(calibs)
+    arr = (Calib * k)(*calibs) if grids is None and 0 < k <= MAX_CAMERAS else None
+    _frame_ids(frame_camera, b, "unproject_cameras: frame_camera")
+    _frame_ids(frame_order, b, "unproject_cameras: frame_order")
+    _call("sceneego_unproject_cameras_f32", feat_cl, feat_cl, grids, arr, int(k), frame_camera, frame_order, b, h, w, c,
+          int(volume_size), C.c_float(cuboid_side), int(img_h), int(img_w), out_f32, out_bf16,
+          C.byref(lay) if lay is not None else None, int(extra_zero_planes))
+
+
+def voxelize_depth_cameras(depth: torch.Tensor, pre_hw, clamp_max: float, rays: torch.Tensor, frame_camera: torch.Tensor,
+                           frame_order: Optional[torch.Tensor], img_h: int, img_w: int, volume_size: int,
+                           cuboid_side: float, occ_f32: Optional[torch.Tensor], occ_bf16: Optional[torch.Tensor],
+                           lay: Optional[VolLayout], channel: int = 0) -> None:
+    """`voxelize_depth_raw` (pre_hw = None and clamp_max = inf: `voxelize_depth`) with a camera per frame: rays
+    (K, img_h, img_w, 3) fp64 stacked tables, frame_camera / frame_order as in `unproject_cameras`."""
+    b, h, w = depth.shape
+    if rays.dim() != 4 or tuple(rays.shape[1:]) != (int(img_h), int(img_w), 3) or rays.dtype != torch.float64:
+        raise SceneEgoError(f"voxelize_depth_cameras: rays must be a (K, {img_h}, {img_w}, 3) float64 tensor")
+    _frame_ids(frame_camera, b, "voxelize_depth_cameras: frame_camera")
+    _frame_ids(frame_order, b, "voxelize_depth_cameras: frame_order")
+    ph, pw = (h, w) if pre_hw is None else (int(pre_hw[0]), int(pre_hw[1]))
+    _call("sceneego_voxelize_depth_cameras_f64", depth, depth, b, h, w, ph, pw, C.c_float(clamp_max), rays,
+          int(rays.shape[0]), frame_camera, frame_order, int(img_h), int(img_w), int(volume_size),
+          C.c_double(cuboid_side), occ_f32, occ_bf16, C.byref(lay) if lay is not None else None, int(channel))
 
 
 def voxelize_depth(depth: torch.Tensor, ray: torch.Tensor, img_h: int, img_w: int, volume_size: int,

@@ -247,6 +247,112 @@ __global__ void __launch_bounds__(320) upsample_pad_kernel(const float* __restri
 // the 512 KB per-frame source stays in L1/L2.  Stores: f32 NCDHW (128 B per warp per
 // channel) and/or bf16 planar padded (512 B per warp per channel group).
 // ---------------------------------------------------------------------------
+// The two halves of unproject_kernel for unproject_cameras_kernel below.  A voxel's geometry: its projection, the four
+// bilinear taps of the virtual image plane and their weights, taps that share a source cell merged (cell -1 = nothing
+// to fetch); frame-invariant for one camera.  Same steps, in the same order, as unproject_kernel, which keeps its own
+// inline copy: calling these helpers from it moved its register allocation (fused form).
+template <bool kProject>
+__device__ __forceinline__ void unproject_taps(const float* __restrict__ grid, const W2CF32& cam, int n, int vx, int vy,
+                                               int vz, int h, int w, float lo, float step, int img_h, int img_w,
+                                               int up_shift_y, int up_shift_x, int (&cell)[4], float (&wt)[4]) {
+  float gx, gy;
+  if (kProject) {
+    float px, py;
+    project_voxel(cam, voxel_coord(lo, step, vx), voxel_coord(lo, step, vy), voxel_coord(0.0f, step, vz), px, py);
+    normalise_px(px, py, img_h, img_w, gx, gy);
+  } else {
+    const float2 g = reinterpret_cast<const float2*>(grid)[n];
+    gx = g.x; gy = g.y;
+  }
+  // ATen grid_sampler_2d, align_corners=True: ix = ((g+1)/2)*(W-1)
+  const float ix = __fmul_rn(__fdiv_rn(__fadd_rn(gx, 1.0f), 2.0f), (float)(img_w - 1));
+  const float iy = __fmul_rn(__fdiv_rn(__fadd_rn(gy, 1.0f), 2.0f), (float)(img_h - 1));
+  const float x0f = floorf(ix), y0f = floorf(iy);
+  const float wx1 = ix - x0f, wy1 = iy - y0f;
+  const float wx0 = (x0f + 1.0f) - ix, wy0 = (y0f + 1.0f) - iy;
+  const int x0 = (int)fminf(fmaxf(x0f, -2.0f), (float)img_w), y0 = (int)fminf(fmaxf(y0f, -2.0f), (float)img_h);   // as in grid_sample_kernel
+  const int pad = (img_w - img_h) / 2;
+
+  // The image plane is the 16x nearest-upsampled source, so the four bilinear taps usually (88 % of the
+  // voxels at V = 64) fall into ONE source cell: taps are merged per source cell and each distinct
+  // 128-byte cell is fetched once (the gather is L2-bandwidth-bound otherwise).
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    const int X = x0 + (t & 1), Y = y0 + (t >> 1);
+    wt[t] = ((t & 1) ? wx1 : wx0) * ((t >> 1) ? wy1 : wy0);
+    const bool inb = (X >= 0) && (X < img_w) && (Y >= 0) && (Y < img_h);   // zeros padding
+    const int xs = X - pad;
+    cell[t] = -1;
+    if (inb && xs >= 0 && xs < img_h) {                                    // outside: ConstantPad2d zeros
+      // nearest source cell: Y * h / img_h.  The 64-bit divisions here (eight per voxel, ~100 instructions each)
+      // were what bounded the kernel; 1024 / 64 is a power of two, otherwise the 32-bit quotient is exact too
+      // (Y * h < 2^31, checked on the host)
+      const int sy = up_shift_y >= 0 ? (Y >> up_shift_y) : (int)((unsigned)(Y * h) / (unsigned)img_h);
+      const int sx = up_shift_x >= 0 ? (xs >> up_shift_x) : (int)((unsigned)(xs * w) / (unsigned)img_h);
+      cell[t] = sy * w + sx;
+    }
+  }
+#pragma unroll
+  for (int t = 1; t < 4; ++t)
+#pragma unroll
+    for (int u = 0; u < t; ++u)
+      if (cell[t] >= 0 && cell[t] == cell[u]) { wt[u] += wt[t]; cell[t] = -1; }
+}
+
+// One frame of one voxel: the merged taps applied to frame b's 32 channels, stored in every requested form.
+__device__ __forceinline__ void unproject_frame(const float* __restrict__ feat, int b, int h, int w, int n, int N, int vx,
+                                                int vy, int vz, const int (&cell)[4], const float (&wt)[4],
+                                                float* __restrict__ out_f32, __nv_bfloat16* __restrict__ out_bf16,
+                                                const sceneego_vol_layout_t& lay, int extra_zero_planes) {
+  constexpr int C = 32;
+  float acc[C];
+#pragma unroll
+  for (int c = 0; c < C; ++c) acc[c] = 0.f;
+  const float* fb = feat + (size_t)b * h * w * C;
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    if (cell[t] >= 0) {
+      // 256-bit loads (sm_100): a warp's lanes fall into ~6 distinct 128-byte source cells, and every load
+      // instruction costs one L1 wavefront per distinct cell whatever its width -- the L1 data pipe, not DRAM,
+      // bounds this kernel (ncu: 80 % of peak with 128-bit loads), so half as many instructions for the same bytes
+      const float* src = fb + (size_t)cell[t] * C;
+      const float w_t = wt[t];
+#pragma unroll
+      for (int q = 0; q < C / 8; ++q) {
+        float v[8];
+        asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                     : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7])
+                     : "l"(src + 8 * q));
+#pragma unroll
+        for (int i = 0; i < 8; ++i) acc[8 * q + i] = fmaf(v[i], w_t, acc[8 * q + i]);
+      }
+    }
+  }
+  if (out_f32) {
+    float* o = out_f32 + (size_t)b * C * N + n;
+#pragma unroll
+    for (int c = 0; c < C; ++c) __stcs(o + (size_t)c * N, acc[c]);
+  }
+  if (out_bf16) {
+    const int64_t cell0 = vol_cell(lay, b, vx, vy, vz, 0, C / 8);
+#pragma unroll
+    for (int g = 0; g < C / 8; ++g) {
+      *reinterpret_cast<uint4*>(out_bf16 + (cell0 + (int64_t)g * lay.plane_stride) * 8) =
+          make_uint4(act_pack2(acc[8 * g + 0], acc[8 * g + 1]), act_pack2(acc[8 * g + 2], acc[8 * g + 3]),
+                     act_pack2(acc[8 * g + 4], acc[8 * g + 5]), act_pack2(acc[8 * g + 6], acc[8 * g + 7]));
+    }
+    // scene-occupancy plane(s) behind the features: cleared here, set by voxelize_kernel
+    if (lay.s2d) {
+      // one cell per 2x2x2 block holds the block's 8 occupancy values: the even-even-even voxel clears it
+      if (extra_zero_planes > 0 && ((vx | vy | vz) & 1) == 0)
+        *reinterpret_cast<uint4*>(out_bf16 + (vol_scene_elem(lay, b, vx, vy, vz, C / 8) & ~(int64_t)7)) = make_uint4(0, 0, 0, 0);
+    } else {
+      for (int g = C / 8; g < C / 8 + extra_zero_planes; ++g)
+        *reinterpret_cast<uint4*>(out_bf16 + (cell0 + (int64_t)g * lay.plane_stride) * 8) = make_uint4(0, 0, 0, 0);
+    }
+  }
+}
+
 template <bool kProject>
 __global__ void __launch_bounds__(128) unproject_kernel(const float* __restrict__ feat, const float* __restrict__ grid,
                                                        W2CF32 cam, int h, int w, int V, float lo, float step,
@@ -357,6 +463,48 @@ __global__ void __launch_bounds__(128) unproject_kernel(const float* __restrict_
     }
   }
   }   // frames
+}
+
+// A camera per frame: frame b is seen through camera frame_camera[b] (grid row frame_camera[b] of the stacked (K,N,2)
+// tables, or coefficient set frame_camera[b] of `cams`).  The block's frame range is taken in `frame_order` (NULL =
+// identity; the host passes a stable sort by camera, so frames that share a camera are adjacent) and a thread
+// recomputes the voxel's geometry only when the camera changes between consecutive frames of its range; the camera is
+// uniform over the block, so the change is too.  Outputs go to the frame's own slot.
+struct W2CSet {
+  W2CF32 k[SCENEEGO_MAX_CAMERAS];
+};
+
+template <bool kProject>
+__global__ void __launch_bounds__(128) unproject_cameras_kernel(const float* __restrict__ feat,
+                                                               const float* __restrict__ grids,
+                                                               const __grid_constant__ W2CSet cams,
+                                                               const int* __restrict__ frame_camera,
+                                                               const int* __restrict__ frame_order, int h, int w, int V,
+                                                               float lo, float step, int img_h, int img_w,
+                                                               float* __restrict__ out_f32,
+                                                               __nv_bfloat16* __restrict__ out_bf16,
+                                                               sceneego_vol_layout_t lay, int extra_zero_planes,
+                                                               int up_shift_y, int up_shift_x, int log2v, int batch,
+                                                               int frames_per_thread) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  const int N = V * V * V;
+  if (n >= N) return;
+  const int vz = log2v >= 0 ? (n & (V - 1)) : n % V;
+  const int vy = log2v >= 0 ? ((n >> log2v) & (V - 1)) : (n / V) % V;
+  const int vx = log2v >= 0 ? (n >> (2 * log2v)) : n / (V * V);
+  int cell[4];
+  float wt[4];
+  int cur = -1;
+  for (int p = blockIdx.y * frames_per_thread; p < min(batch, (int)(blockIdx.y + 1) * frames_per_thread); ++p) {
+    const int b = frame_order ? __ldg(frame_order + p) : p;
+    const int k = __ldg(frame_camera + b);
+    if (k != cur) {
+      cur = k;
+      unproject_taps<kProject>(kProject ? grids : grids + (size_t)k * N * 2, cams.k[k], n, vx, vy, vz, h, w, lo, step, img_h, img_w,
+                               up_shift_y, up_shift_x, cell, wt);
+    }
+    unproject_frame(feat, b, h, w, n, N, vx, vy, vz, cell, wt, out_f32, out_bf16, lay, extra_zero_planes);
+  }
 }
 
 // ---------------------------------------------------------------------------
@@ -521,6 +669,92 @@ __global__ void __launch_bounds__(256) voxelize_kernel(const float* __restrict__
     // one thread per block writes the zero-depth voxel when any pixel of the block has zero depth (a per-warp vote
     // instead of the block-wide one made 8x more writers hammer the same voxel: 3.6 -> 4.6 us); block (0,0,z) also
     // does it for the padded columns
+    const bool any_zero = __syncthreads_or(zero ? 1 : 0) != 0 || (pad > 0 && blockIdx.x == 0 && blockIdx.y == 0);
+    if (any_zero && threadIdx.x == 0 && q0_in) {
+      const int c = (int)q0;
+      if (occ_f32) occ_f32[(((size_t)b * V + c) * V + c) * V] = 1.0f;
+      if (occ_bf16) set_occupied(occ_bf16, lay, b, c, c, 0, channel, V);
+    }
+    if (ix >= 0) {
+      if (occ_f32) occ_f32[(((size_t)b * V + ix) * V + iy) * V + iz] = 1.0f;
+      if (occ_bf16) set_occupied(occ_bf16, lay, b, ix, iy, iz, channel, V);
+    }
+  }
+}
+
+// A camera per frame: frame b back-projects through ray table frame_camera[b] of the stacked (K, img_h, img_w, 3) tables.
+// The block's frames are taken in `frame_order` (NULL = identity; a stable sort by camera from the host), and the
+// pixel's ray is reloaded only when the camera changes, so a table is still fetched once per block and camera run.  The
+// fp64 steps are voxelize_kernel's (quantize_point performs them in the same order: ray * depth, + s/2, * V, / s).
+// Eight blocks per SM on the power-of-two paths (32 registers, as voxelize_kernel gets): the frame order and the camera
+// ids add two dependent loads in front of the ray's, and occupancy is what hides them.
+template <int kPow2Side>
+__global__ void __launch_bounds__(256, kPow2Side ? 8 : 1) voxelize_cameras_kernel(const float* __restrict__ depth, int h, int w,
+                                                              NearestMaps nm, const double* __restrict__ rays,
+                                                              const int* __restrict__ frame_camera,
+                                                              const int* __restrict__ frame_order, int img_h, int img_w,
+                                                              int V, double side, double inv_side,
+                                                              float* __restrict__ occ_f32,
+                                                              __nv_bfloat16* __restrict__ occ_bf16,
+                                                              sceneego_vol_layout_t lay, int channel, int batch,
+                                                              int frames_per_block, int cols) {
+  const int xs = blockIdx.x * blockDim.x + threadIdx.x;
+  const int Y = blockIdx.y;
+  const int pad = (img_w - cols) / 2;
+  const int X = xs + pad;
+  const bool in_src = xs < cols;
+  int sy = (int)floor(__dmul_rn((double)Y, nm.ify1));
+  int sx = (int)floor(__dmul_rn((double)(in_src ? xs : 0), nm.ifx1));
+  sy = sy < nm.pre_h - 1 ? sy : nm.pre_h - 1;
+  sx = sx < nm.pre_w - 1 ? sx : nm.pre_w - 1;
+  sy = (int)floor(__dmul_rn((double)sy, nm.ify0));
+  sx = (int)floor(__dmul_rn((double)sx, nm.ifx0));
+  sy = sy < h - 1 ? sy : h - 1;
+  sx = sx < w - 1 ? sx : w - 1;
+  const double half = side / 2;
+  const double Vd = (double)V;
+  const double hi = (double)(V - 1);
+  const double q0 = rint(kPow2Side ? __dmul_rn(__dmul_rn(half, Vd), inv_side) : __ddiv_rn(__dmul_rn(half, Vd), side));
+  const bool q0_in = q0 >= 0.0 && q0 <= hi;
+  const int b_begin = blockIdx.z * frames_per_block;
+  constexpr int kMaxFpb = 8;
+  int fb[kMaxFpb], fk[kMaxFpb];
+  float dvs[kMaxFpb];
+#pragma unroll
+  for (int f = 0; f < kMaxFpb; ++f) {
+    dvs[f] = 0.f;
+    fb[f] = -1; fk[f] = 0;
+    if (f < frames_per_block && b_begin + f < batch) {
+      fb[f] = frame_order ? __ldg(frame_order + b_begin + f) : b_begin + f;
+      fk[f] = __ldg(frame_camera + fb[f]);
+      if (in_src) {
+        const float t = __ldcs(depth + ((size_t)fb[f] * h + sy) * w + sx);
+        dvs[f] = t > nm.clamp_max ? nm.clamp_max : t;          // NaN compares false and stays, like NumPy's mask
+      }
+    }
+  }
+  int cur = -1;
+  double r0 = 0.0, r1 = 0.0, r2 = 0.0;
+#pragma unroll
+  for (int f = 0; f < kMaxFpb; ++f) {
+    const int b = fb[f];
+    if (b < 0) break;                                        // uniform over the block
+    if (fk[f] != cur) {                                      // uniform over the block as well
+      cur = fk[f];
+      if (in_src) {
+        const double* r = rays + ((size_t)cur * img_h * img_w + (size_t)Y * img_w + X) * 3;
+        r0 = r[0]; r1 = r[1]; r2 = r[2];
+      }
+    }
+    const float dv = dvs[f];
+    int ix = -1, iy = 0, iz = 0;
+    const bool zero = in_src && (dv == 0.0f);
+    if (in_src && !zero) {
+      const double d = (double)dv;
+      if (!quantize_point<kPow2Side>(__dmul_rn(r0, d), __dmul_rn(r1, d), __dmul_rn(r2, d), half, Vd, side, inv_side, hi,
+                                     ix, iy, iz))
+        ix = -1;
+    }
     const bool any_zero = __syncthreads_or(zero ? 1 : 0) != 0 || (pad > 0 && blockIdx.x == 0 && blockIdx.y == 0);
     if (any_zero && threadIdx.x == 0 && q0_in) {
       const int c = (int)q0;
@@ -833,11 +1067,12 @@ extern "C" int sceneego_features_upsample_pad_f32(const float* d_in, float* d_ou
   return SCENEEGO_OK;
 }
 
-extern "C" int sceneego_unproject_f32(const float* d_feat, const float* d_grid, const sceneego_calib_t* calib,
-                                      int batch, int h, int w, int c, int V, float side, int img_h, int img_w,
-                                      float* d_out_f32, void* d_out_bf16, const sceneego_vol_layout_t* lay,
-                                      int extra_zero_planes, void* stream) {
-  SE_REQUIRE(d_feat && (d_grid || calib) && (d_out_f32 || d_out_bf16), "unproject: null argument");
+// d_frame_camera == NULL: one camera (d_grid, or calibs[0] when d_grid is NULL) for the whole batch
+static int unproject_impl(const float* d_feat, const float* d_grid, const sceneego_calib_t* calibs, int n_cameras,
+                          const int32_t* d_frame_camera, const int32_t* d_frame_order, int batch, int h, int w, int c,
+                          int V, float side, int img_h, int img_w, float* d_out_f32, void* d_out_bf16,
+                          const sceneego_vol_layout_t* lay, int extra_zero_planes, void* stream) {
+  SE_REQUIRE(d_feat && (d_grid || calibs) && (d_out_f32 || d_out_bf16), "unproject: null argument");
   SE_REQUIRE(c == 32, "unproject: 32 feature channels expected (process_features output)");
   SE_REQUIRE(!d_out_bf16 || (lay && (lay->s2d ? 2 * lay->side : lay->side) == V), "unproject: bf16 output needs a matching layout");
   SE_REQUIRE(batch > 0 && batch <= 65535 && img_w >= img_h, "unproject: bad batch / image plane");
@@ -847,7 +1082,6 @@ extern "C" int sceneego_unproject_f32(const float* d_feat, const float* d_grid, 
   sceneego_vol_layout_t L = lay ? *lay : sceneego_vol_layout_t{};
   const float step = (float)((double)side / (V - 1));
   const float lo = (float)(-(double)side / 2);
-  W2CF32 cam = calib ? make_w2c(calib) : W2CF32{};
   SE_REQUIRE(h > 0 && w > 0 && (long long)img_w * (h > w ? h : w) < (1ll << 31), "unproject: image plane too large");
   auto shift_of = [](int num, int den) {       // log2(num / den) when that ratio is an exact power of two, else -1
     if (den <= 0 || num % den) return -1;
@@ -856,22 +1090,59 @@ extern "C" int sceneego_unproject_f32(const float* d_feat, const float* d_grid, 
     return -1;
   };
   const int sh_y = shift_of(img_h, h), sh_x = shift_of(img_h, w), log2v = shift_of(V, 1);
-  if (d_grid)
-    unproject_kernel<false><<<grid, 128, 0, (cudaStream_t)stream>>>(d_feat, d_grid, cam, h, w, V, lo, step, img_h,
-                                                                    img_w, d_out_f32, (__nv_bfloat16*)d_out_bf16, L,
-                                                                    extra_zero_planes, sh_y, sh_x, log2v, batch, fpt);
-  else
-    unproject_kernel<true><<<grid, 128, 0, (cudaStream_t)stream>>>(d_feat, nullptr, cam, h, w, V, lo, step, img_h,
-                                                                   img_w, d_out_f32, (__nv_bfloat16*)d_out_bf16, L,
-                                                                   extra_zero_planes, sh_y, sh_x, log2v, batch, fpt);
+  cudaStream_t st = (cudaStream_t)stream;
+  __nv_bfloat16* o16 = (__nv_bfloat16*)d_out_bf16;
+  if (d_frame_camera) {
+    W2CSet cams{};
+    if (!d_grid)
+      for (int k = 0; k < n_cameras; ++k) cams.k[k] = make_w2c(calibs + k);
+    if (d_grid)
+      unproject_cameras_kernel<false><<<grid, 128, 0, st>>>(d_feat, d_grid, cams, d_frame_camera, d_frame_order, h, w, V,
+                                                            lo, step, img_h, img_w, d_out_f32, o16, L,
+                                                            extra_zero_planes, sh_y, sh_x, log2v, batch, fpt);
+    else
+      unproject_cameras_kernel<true><<<grid, 128, 0, st>>>(d_feat, nullptr, cams, d_frame_camera, d_frame_order, h, w, V,
+                                                           lo, step, img_h, img_w, d_out_f32, o16, L,
+                                                           extra_zero_planes, sh_y, sh_x, log2v, batch, fpt);
+  } else {
+    W2CF32 cam = calibs ? make_w2c(calibs) : W2CF32{};
+    if (d_grid)
+      unproject_kernel<false><<<grid, 128, 0, st>>>(d_feat, d_grid, cam, h, w, V, lo, step, img_h, img_w, d_out_f32, o16,
+                                                    L, extra_zero_planes, sh_y, sh_x, log2v, batch, fpt);
+    else
+      unproject_kernel<true><<<grid, 128, 0, st>>>(d_feat, nullptr, cam, h, w, V, lo, step, img_h, img_w, d_out_f32, o16,
+                                                   L, extra_zero_planes, sh_y, sh_x, log2v, batch, fpt);
+  }
   SE_CUDA_LAUNCH_CHECK("unproject");
   return SCENEEGO_OK;
 }
 
+extern "C" int sceneego_unproject_f32(const float* d_feat, const float* d_grid, const sceneego_calib_t* calib,
+                                      int batch, int h, int w, int c, int V, float side, int img_h, int img_w,
+                                      float* d_out_f32, void* d_out_bf16, const sceneego_vol_layout_t* lay,
+                                      int extra_zero_planes, void* stream) {
+  return unproject_impl(d_feat, d_grid, calib, 1, nullptr, nullptr, batch, h, w, c, V, side, img_h, img_w, d_out_f32,
+                        d_out_bf16, lay, extra_zero_planes, stream);
+}
+
+extern "C" int sceneego_unproject_cameras_f32(const float* d_feat, const float* d_grids, const sceneego_calib_t* calibs,
+                                              int n_cameras, const int32_t* d_frame_camera,
+                                              const int32_t* d_frame_order, int batch, int h, int w, int c, int V,
+                                              float side, int img_h, int img_w, float* d_out_f32, void* d_out_bf16,
+                                              const sceneego_vol_layout_t* lay, int extra_zero_planes, void* stream) {
+  SE_REQUIRE(n_cameras >= 1 && n_cameras <= SCENEEGO_MAX_CAMERAS, "unproject_cameras: n_cameras must be in [1, %d]",
+             SCENEEGO_MAX_CAMERAS);
+  SE_REQUIRE(d_frame_camera, "unproject_cameras: null frame_camera");
+  return unproject_impl(d_feat, d_grids, calibs, n_cameras, d_frame_camera, d_frame_order, batch, h, w, c, V, side,
+                        img_h, img_w, d_out_f32, d_out_bf16, lay, extra_zero_planes, stream);
+}
+
+// d_frame_camera != NULL: d_ray holds one table per camera, frame b uses table d_frame_camera[b]
 static int voxelize_impl(const float* d_depth, int batch, int h, int w, int pre_h, int pre_w, float clamp_max,
                          const double* d_ray, int img_h, int img_w, int V, double side, float* d_occ_f32,
                          void* d_occ_bf16, const sceneego_vol_layout_t* lay, int channel, void* stream,
-                         bool direct = false) {
+                         bool direct = false, const int32_t* d_frame_camera = nullptr,
+                         const int32_t* d_frame_order = nullptr) {
   SE_REQUIRE(d_depth && d_ray && (d_occ_f32 || d_occ_bf16), "voxelize: null argument");
   SE_REQUIRE(batch > 0 && batch <= 65535 && h > 0 && w > 0 && pre_h > 0 && pre_w > 0 && img_w >= img_h, "voxelize: bad shape");
   SE_REQUIRE(!d_occ_bf16 || (lay && (lay->s2d ? 2 * lay->side : lay->side) == V && channel >= 0), "voxelize: bf16 output needs a matching layout");
@@ -891,15 +1162,31 @@ static int voxelize_impl(const float* d_depth, int batch, int h, int w, int pre_
   int e2 = 0;
   const bool pow2 = side > 0 && frexp(side, &e2) == 0.5;       // side == 2^(e2-1): divide == exact multiply
   const bool pow2_v = V > 0 && (V & (V - 1)) == 0;
-  if (pow2 && pow2_v)
-    voxelize_kernel<2><<<grid, 256, 0, (cudaStream_t)stream>>>(d_depth, h, w, nm, d_ray, img_h, img_w, V, side, 1.0 / side,
-                                                               d_occ_f32, (__nv_bfloat16*)d_occ_bf16, L, channel, batch, fpb, cols);
-  else if (pow2)
-    voxelize_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(d_depth, h, w, nm, d_ray, img_h, img_w, V, side, 1.0 / side,
-                                                               d_occ_f32, (__nv_bfloat16*)d_occ_bf16, L, channel, batch, fpb, cols);
-  else
-    voxelize_kernel<0><<<grid, 256, 0, (cudaStream_t)stream>>>(d_depth, h, w, nm, d_ray, img_h, img_w, V, side, 0.0,
-                                                                   d_occ_f32, (__nv_bfloat16*)d_occ_bf16, L, channel, batch, fpb, cols);
+  cudaStream_t st = (cudaStream_t)stream;
+  __nv_bfloat16* o16 = (__nv_bfloat16*)d_occ_bf16;
+  const int path = pow2 && pow2_v ? 2 : pow2 ? 1 : 0;
+  const double inv = pow2 ? 1.0 / side : 0.0;
+  if (d_frame_camera) {
+    if (path == 2)
+      voxelize_cameras_kernel<2><<<grid, 256, 0, st>>>(d_depth, h, w, nm, d_ray, d_frame_camera, d_frame_order, img_h,
+                                                       img_w, V, side, inv, d_occ_f32, o16, L, channel, batch, fpb, cols);
+    else if (path == 1)
+      voxelize_cameras_kernel<1><<<grid, 256, 0, st>>>(d_depth, h, w, nm, d_ray, d_frame_camera, d_frame_order, img_h,
+                                                       img_w, V, side, inv, d_occ_f32, o16, L, channel, batch, fpb, cols);
+    else
+      voxelize_cameras_kernel<0><<<grid, 256, 0, st>>>(d_depth, h, w, nm, d_ray, d_frame_camera, d_frame_order, img_h,
+                                                       img_w, V, side, inv, d_occ_f32, o16, L, channel, batch, fpb, cols);
+  } else {
+    if (path == 2)
+      voxelize_kernel<2><<<grid, 256, 0, st>>>(d_depth, h, w, nm, d_ray, img_h, img_w, V, side, inv, d_occ_f32, o16, L,
+                                               channel, batch, fpb, cols);
+    else if (path == 1)
+      voxelize_kernel<1><<<grid, 256, 0, st>>>(d_depth, h, w, nm, d_ray, img_h, img_w, V, side, inv, d_occ_f32, o16, L,
+                                               channel, batch, fpb, cols);
+    else
+      voxelize_kernel<0><<<grid, 256, 0, st>>>(d_depth, h, w, nm, d_ray, img_h, img_w, V, side, inv, d_occ_f32, o16, L,
+                                               channel, batch, fpb, cols);
+  }
   SE_CUDA_LAUNCH_CHECK("voxelize");
   return SCENEEGO_OK;
 }
@@ -918,6 +1205,19 @@ extern "C" int sceneego_voxelize_depth_raw_f64(const float* d_depth_raw, int bat
                                                const sceneego_vol_layout_t* lay, int channel, void* stream) {
   return voxelize_impl(d_depth_raw, batch, h, w, pre_h, pre_w, clamp_max, d_ray, img_h, img_w, V, side, d_occ_f32,
                        d_occ_bf16, lay, channel, stream);
+}
+
+extern "C" int sceneego_voxelize_depth_cameras_f64(const float* d_depth, int batch, int h, int w, int pre_h, int pre_w,
+                                                   float clamp_max, const double* d_rays, int n_cameras,
+                                                   const int32_t* d_frame_camera, const int32_t* d_frame_order,
+                                                   int img_h, int img_w, int V, double side, float* d_occ_f32,
+                                                   void* d_occ_bf16, const sceneego_vol_layout_t* lay, int channel,
+                                                   void* stream) {
+  SE_REQUIRE(n_cameras >= 1 && n_cameras <= SCENEEGO_MAX_CAMERAS, "voxelize_cameras: n_cameras must be in [1, %d]",
+             SCENEEGO_MAX_CAMERAS);
+  SE_REQUIRE(d_frame_camera, "voxelize_cameras: null frame_camera");
+  return voxelize_impl(d_depth, batch, h, w, pre_h, pre_w, clamp_max, d_rays, img_h, img_w, V, side, d_occ_f32,
+                       d_occ_bf16, lay, channel, stream, false, d_frame_camera, d_frame_order);
 }
 
 extern "C" int sceneego_voxelize_depth_dataset_f64(const float* d_depth_raw, int batch, int h, int w, int pre_h, int pre_w,

@@ -8,7 +8,9 @@ C-ABI of include/sceneego_b200.h:
     process_features (1x1 conv; the x16 upsample + pad are never materialised
                       unless `materialize_features`)      -> sceneego_feature_conv1x1_f32
     unproject_heatmaps_one_view_batch + torch.cat         -> sceneego_unproject_f32
+                          (a camera per frame, camera_ids=) -> sceneego_unproject_cameras_f32
     depth_map_to_voxel_numpy loop (host NumPy in the ref) -> sceneego_voxelize_depth_f64
+                          (a camera per frame, camera_ids=) -> sceneego_voxelize_depth_cameras_f64
     point_cloud_to_voxel_numpy (clouds for scene_volumes=) -> sceneego_voxelize_points
     scan_to_voxels (world scan + B poses, scene_volumes=)   -> sceneego_voxelize_scan
     volume_net (V2VModel)                                 -> sceneego_v2v_run
@@ -40,6 +42,53 @@ def _resolve_calibration(path):
     if os.path.exists(alt):
         return alt
     raise FileNotFoundError(path)
+
+
+def _camera_model(calibration, size, n_cameras):
+    """`add_camera`'s host-side checks: a calibration file path or a FishEyeCameraCalibrated whose image size is the
+    module's (image_width, image_height), and room for one more camera."""
+    if n_cameras >= _lib.MAX_CAMERAS:
+        raise _lib.SceneEgoError(f"a module holds at most {_lib.MAX_CAMERAS} cameras")
+    if isinstance(calibration, FishEyeCameraCalibrated):
+        model = calibration
+    elif isinstance(calibration, (str, os.PathLike)):
+        model = FishEyeCameraCalibrated(calibration_file_path=_resolve_calibration(os.fspath(calibration)))
+    else:
+        raise _lib.SceneEgoError(f"add_camera takes a calibration file path or a FishEyeCameraCalibrated, got "
+                                 f"{type(calibration).__name__}")
+    got = tuple(int(v) for v in np.asarray(model.img_size).reshape(-1))
+    if got != tuple(size):
+        raise _lib.SceneEgoError(f"camera image size {got} differs from the module's (image_width, image_height) "
+                                 f"{tuple(size)}: the feature map's crop and squash assume the module's size")
+    return model
+
+
+def camera_ids_host(camera_ids, b, n_cameras):
+    """`camera_ids` of lift() / forward() -> (B,) int32 NumPy array.  Host-side only (a list, a NumPy array or a CPU
+    tensor of integers): ids on the device could only be checked after a synchronisation."""
+    if isinstance(camera_ids, torch.Tensor):
+        if camera_ids.device.type != "cpu":
+            raise _lib.SceneEgoError("camera_ids must be a host-side sequence (list, NumPy array or CPU tensor), got a "
+                                     f"tensor on {camera_ids.device}: checking device ids would need a synchronisation")
+        if camera_ids.dtype == torch.bool or camera_ids.dtype.is_floating_point or camera_ids.dtype.is_complex:
+            raise _lib.SceneEgoError(f"camera_ids must be integers, got {camera_ids.dtype}")
+        a = camera_ids.numpy()
+    else:
+        a = np.asarray(camera_ids)
+    if a.dtype.kind not in "iu":
+        raise _lib.SceneEgoError(f"camera_ids must be integers, got {a.dtype}")
+    if a.shape != (b,):
+        raise _lib.SceneEgoError(f"camera_ids must hold one id per frame ({b}), got shape {a.shape}")
+    if a.min() < 0 or a.max() >= n_cameras:
+        raise _lib.SceneEgoError(f"camera_ids must lie in [0, {n_cameras}) (cameras come from add_camera), got "
+                                 f"[{a.min()}, {a.max()}]")
+    return a.astype(np.int32)
+
+
+def camera_frame_order(ids):
+    """Stable sort of the frames by camera: the order the camera-per-frame kernels visit frames in, so that frames
+    that share a camera are adjacent and a voxel's geometry (a pixel's ray) is reloaded once per run."""
+    return np.argsort(np.asarray(ids), kind="stable").astype(np.int32)
 
 
 class VoxelNetwork_depth(nn.Module):
@@ -138,6 +187,12 @@ class VoxelNetwork_depth(nn.Module):
         # ray table: device copy row-major for the kernel, NumPy x-major copy for API parity
         self._ray_dev = self.fisheye_camera_model.ray_table_device(self.image_width, self.image_height, dev)
         self.ray = self._ray_dev.permute(1, 0, 2).reshape(-1, 3).cpu().numpy()
+        # cameras for camera_ids= (add_camera); camera 0 is the config's.  The stacked (K,N,2) grids and
+        # (K,H,W,3) ray tables are built when first needed and rebuilt (new storage) by add_camera
+        self.cameras = [self.fisheye_camera_model]
+        self._cam_calibs = [self._calib]
+        self._cam_grids = None
+        self._cam_rays = None
         cv = self.coord_volume
         self._axis = torch.stack([cv[:, 0, 0, 0], cv[0, :, 0, 1], cv[0, 0, :, 2]]).contiguous()
         self.last_launches = 0
@@ -161,6 +216,57 @@ class VoxelNetwork_depth(nn.Module):
         az = 0.0 + step * idx
         gx, gy, gz = torch.meshgrid(axy, axy, az, indexing='ij')
         return torch.stack([gx, gy, gz], dim=-1).contiguous()
+
+    # ------------------------------------------------------------------ cameras
+    def add_camera(self, calibration) -> int:
+        """Set up one more fisheye camera for `camera_ids=` and return its id.  `calibration` is a calibration file path
+        or a FishEyeCameraCalibrated of the module's image size.  Its calib struct, table-mode grid and ray table are
+        built by the functions the constructor uses, so frames of this camera lift exactly as they would through a
+        module built from that file.  The reference attributes (ray, grid_coord_proj_batch, ...) stay camera 0's."""
+        model = _camera_model(calibration, (self.image_width, self.image_height), len(self.cameras))
+        dev = _lib._as_device(self.device)
+        grid_px = op.get_projected_2d_points_with_coord_volumes(fisheye_model=model, coord_volume=self.coord_volume)
+        grid = op.get_grid_coord_proj_batch(grid_px, batch_size=1, heatmap_shape=self.heatmap_shape)
+        grid = grid[0].reshape(-1, 2).contiguous().float()
+        ray = model.ray_table_device(self.image_width, self.image_height, dev)
+        grids, rays = self._camera_tables()
+        self._cam_grids = torch.cat([grids, grid.unsqueeze(0)])
+        self._cam_rays = torch.cat([rays, ray.unsqueeze(0)])
+        self._cam_calibs.append(model.calib_struct(self.image_width, self.image_height))
+        self.cameras.append(model)
+        return len(self.cameras) - 1
+
+    def _camera_tables(self):
+        """(K,N,2) f32 table-mode grids and (K,H,W,3) fp64 ray tables of the cameras, camera 0 first."""
+        if self._cam_grids is None:
+            self._cam_grids = self._grid_table(self.grid_coord_proj_batch, 1).unsqueeze(0)
+            self._cam_rays = self._ray_dev.unsqueeze(0)
+        return self._cam_grids, self._cam_rays
+
+    def _camera_ids(self, camera_ids, grid_coord_proj_batch, b):
+        """Checked host ids, or None.  Per-camera grids come from add_camera, so the grid argument must be the
+        module's own table."""
+        if camera_ids is None:
+            return None
+        ids = camera_ids_host(camera_ids, b, len(self.cameras))
+        own, g = self.grid_coord_proj_batch, grid_coord_proj_batch
+        if g is not own and not (isinstance(g, torch.Tensor) and g.dtype == own.dtype and g.device == own.device
+                                 and g.data_ptr() == own.data_ptr() and g.shape[1:] == own.shape[1:]
+                                 and g.stride() == own.stride()):
+            raise _lib.SceneEgoError("with camera_ids, grid_coord_proj_batch must be the module's own table: the "
+                                     "per-camera tables come from add_camera")
+        self._camera_tables()
+        return ids
+
+    @staticmethod
+    def _camera_host(ids, chunk):
+        """ids and, per V2V chunk, the chunk's stable frame order (chunk-local indices) as one pinned (2B,) int32
+        tensor [ids | order], so that its copy to the device needs no synchronisation."""
+        b = ids.shape[0]
+        h = torch.empty(2 * b, dtype=torch.int32, pin_memory=True)
+        h.numpy()[:b] = ids
+        h.numpy()[b:] = np.concatenate([camera_frame_order(ids[s:s + chunk]) for s in range(0, b, chunk)])
+        return h
 
     # ------------------------------------------------------------------ argument handling
     def _grid_table(self, grid_coord_proj_batch, b):
@@ -207,9 +313,11 @@ class VoxelNetwork_depth(nn.Module):
 
     # ------------------------------------------------------------------ hot path
     def lift(self, backbone_features, grid_coord_proj_batch, coord_volumes=None, scene_volumes=None,
-             depth_map_batch=None):
+             depth_map_batch=None, camera_ids=None):
         """Everything the reference forward does after `self.backbone(images)`
-        (network/voxel_net_depth.py:237-273)."""
+        (network/voxel_net_depth.py:237-273).  camera_ids: None (every frame through camera 0, the config's), or one
+        camera id per frame (a list, NumPy array or CPU tensor of ints in [0, len(self.cameras))): frame b is lifted
+        exactly as a module built from camera camera_ids[b]'s calibration would lift it in the same batch."""
         if self.training:
             raise _lib.SceneEgoError("VoxelNetwork_depth is inference-only (BatchNorm is folded from the running "
                                      "statistics): call .eval() first, like demo.py:32 / test.py:29")
@@ -219,17 +327,18 @@ class VoxelNetwork_depth(nn.Module):
         conv = self.process_features[0]
         return self._lift_feat32(lambda out: _lib.feature_conv1x1(feat, conv.weight, conv.bias, out=out),
                                  feat.shape[0], (feat.shape[2], feat.shape[3]), feat.device, 1,
-                                 grid_coord_proj_batch, coord_volumes, scene_volumes, depth_map_batch)
+                                 grid_coord_proj_batch, coord_volumes, scene_volumes, depth_map_batch, camera_ids)
 
     def _lift_feat32(self, make_feat32, b, hw, dev, feat_launches, grid_coord_proj_batch, coord_volumes, scene_volumes,
-                     depth_map_batch):
+                     depth_map_batch, camera_ids=None):
         """The stage from `feat32` on.  `make_feat32(out)` produces the (B,h,w,32) channel-last f32 map of
         process_features[0] -- from the backbone's 256-channel features (lift) or fused with the backbone's last
         deconvolution (forward with backbone_handoff=True) -- into `out` (None: a fresh tensor)."""
         v = self.volume_size
+        ids = self._camera_ids(camera_ids, grid_coord_proj_batch, b)
         if b <= self.graph_max_batch and self._graphs is not None:
             out = self._lift_graphed(make_feat32, b, hw, dev, feat_launches, grid_coord_proj_batch, coord_volumes,
-                                     scene_volumes, depth_map_batch)
+                                     scene_volumes, depth_map_batch, ids)
             if out is not NotImplemented:
                 return out
         feat32 = make_feat32(None)                                            # (B,64,64,32) channel-last
@@ -273,12 +382,14 @@ class VoxelNetwork_depth(nn.Module):
         vn = self.volume_net
         pg = vn.program(v, min(vn.max_chunk, b), dev)
         chunk = pg.chunk
+        cam = None if ids is None else self._camera_host(ids, chunk).to(dev, non_blocking=True)
         logits = torch.empty(b, self.num_joints, v, v, v, dtype=torch.float32, device=dev)
         for s in range(0, b, chunk):
             n = min(chunk, b - s)
             launches += self._fill_v2v_input(pg, feat32[s:s + n], grid,
                                              None if scene_volumes is None else scene_volumes[s:s + n],
-                                             None if depth_map_batch is None else depth_map_batch[s:s + n])
+                                             None if depth_map_batch is None else depth_map_batch[s:s + n],
+                                             None if cam is None else (cam[s:s + n], cam[b + s:b + s + n]))
             launches += vn.run_chunk(pg, n, logits[s:s + n])
         kp, volumes = _lib.softargmax3d(logits, float(self.volume_multiplier), bool(self.volume_softmax),
                                         self._axis if coords is None else None, coords, self.materialize_volumes)
@@ -290,7 +401,7 @@ class VoxelNetwork_depth(nn.Module):
         return kp, features, volumes, self.coord_volumes
 
     def _lift_graphed(self, make_feat32, b, hw, dev, feat_launches, grid_coord_proj_batch, coord_volumes, scene_volumes,
-                      depth_map_batch):
+                      depth_map_batch, ids=None):
         """Small batches (demo.py runs batch 1): the ~68 launches from the gather to the V2V logits replay as ONE
         captured CUDA graph over static buffers; the 1x1 feature conv (live weights), the copy of the scene input
         into its static buffer, the soft-argmax and outputs #2 / #3 (fresh tensors) stay outside the graph.
@@ -311,8 +422,11 @@ class VoxelNetwork_depth(nn.Module):
             src = src.reshape((b,) + tuple(src.shape[-3:] if kind == "scene" else src.shape[-2:]))
             if kind == "scene" and self.with_intersection:
                 return NotImplemented                       # the eager path raises the explanatory error
+        # camera mode: the ids and frame order live in a static buffer refilled before every replay, so a new
+        # assignment replays the same capture; add_camera reallocates the stacked tables, which recaptures
+        cams = None if ids is None else (self._cam_grids.data_ptr(), self._cam_rays.data_ptr())
         key = (b, kind, None if src is None else tuple(src.shape), bool(self.fused_projection),
-               0 if grid is None else grid.data_ptr(), self.depth_preprocess, id(pg), dev.index)
+               0 if grid is None else grid.data_ptr(), self.depth_preprocess, id(pg), dev.index, cams)
         g = self._graphs.get(key)
         main = torch.cuda.current_stream(dev)
         if g is None:
@@ -321,15 +435,19 @@ class VoxelNetwork_depth(nn.Module):
             g = {"pg": pg, "grid": grid,
                  "feat32": torch.empty(b, hw[0], hw[1], 32, dtype=torch.float32, device=dev),
                  "src": None if src is None else torch.empty(src.shape, dtype=torch.float32, device=dev),
-                 "logits": torch.empty(b, self.num_joints, v, v, v, dtype=torch.float32, device=dev)}
+                 "logits": torch.empty(b, self.num_joints, v, v, v, dtype=torch.float32, device=dev),
+                 "cam": None if ids is None else torch.empty(2 * b, dtype=torch.int32, device=dev)}
 
             def body():
                 n = self._fill_v2v_input(pg, g["feat32"], grid, g["src"] if kind == "scene" else None,
-                                         g["src"] if kind == "depth" else None)
+                                         g["src"] if kind == "depth" else None,
+                                         None if ids is None else (g["cam"][:b], g["cam"][b:]))
                 return n + vn.run_chunk(pg, b, g["logits"])
             make_feat32(g["feat32"])
             if src is not None:
                 g["src"].copy_(src)
+            if ids is not None:
+                g["cam"].copy_(self._camera_host(ids, b), non_blocking=True)
             body()                                          # eager warm-up: per-device kernel attributes get set
             main.synchronize()
             graph = torch.cuda.CUDAGraph()
@@ -340,6 +458,8 @@ class VoxelNetwork_depth(nn.Module):
         make_feat32(g["feat32"])
         if src is not None:
             g["src"].copy_(src)
+        if ids is not None:
+            g["cam"].copy_(self._camera_host(ids, b), non_blocking=True)
         features, feat_done = None, None
         if self.materialize_features:
             side = self._side_streams.get(dev)
@@ -361,15 +481,21 @@ class VoxelNetwork_depth(nn.Module):
         self.last_logits = g["logits"].clone() if self.keep_logits else None
         return kp, features, volumes, self.coord_volumes
 
-    def _fill_v2v_input(self, pg, feat32, grid, scene_volumes, depth_map_batch) -> int:
+    def _fill_v2v_input(self, pg, feat32, grid, scene_volumes, depth_map_batch, cams=None) -> int:
         """a2 + a5 + a6: write the lifted features and the scene occupancy of `n` frames straight into the V2V
-        program's input buffer (network/voxel_net_depth.py:243-262).  Returns the number of kernels launched."""
+        program's input buffer (network/voxel_net_depth.py:243-262).  cams: None (camera 0) or the (n,) int32 device
+        camera ids and chunk-local frame order of the frames.  Returns the number of kernels launched."""
         n = feat32.shape[0]
         v = self.volume_size
         in_buf = pg.buffers[pg.in_buf]
         img_h, img_w = self.heatmap_shape
-        _lib.unproject(feat32, grid, self._calib if self.fused_projection else None, v, float(self.cuboid_side),
-                       img_h, img_w, None, in_buf, pg.lay_in, extra_zero_planes=pg.extra_zero_planes)
+        if cams is None:
+            _lib.unproject(feat32, grid, self._calib if self.fused_projection else None, v, float(self.cuboid_side),
+                           img_h, img_w, None, in_buf, pg.lay_in, extra_zero_planes=pg.extra_zero_planes)
+        else:
+            _lib.unproject_cameras(feat32, None if self.fused_projection else self._cam_grids, self._cam_calibs, cams[0],
+                                   cams[1], v, float(self.cuboid_side), img_h, img_w, None, in_buf, pg.lay_in,
+                                   extra_zero_planes=pg.extra_zero_planes)
         launches = 1
         if self.with_scene is True:
             scene_ch = 64 if self.with_intersection else 32
@@ -387,7 +513,13 @@ class VoxelNetwork_depth(nn.Module):
                 # one pass builds the whole occupancy plane from it and leaves the grid zero for the next batch
                 scratch = pg.occ_scratch[:n] if pg.zwin else None
                 dst_bf16 = None if pg.zwin else in_buf
-                if self.depth_preprocess is not None:
+                if cams is not None:
+                    pre, cm = (None, float("inf")) if self.depth_preprocess is None else \
+                        (self.depth_preprocess[:2], float(self.depth_preprocess[2]))
+                    _lib.voxelize_depth_cameras(d, pre, cm, self._cam_rays, cams[0], cams[1], self.image_height,
+                                                self.image_width, v, float(self.cuboid_side), scratch, dst_bf16,
+                                                pg.lay_in, channel=scene_ch)
+                elif self.depth_preprocess is not None:
                     ph, pw, cm = self.depth_preprocess
                     _lib.voxelize_depth_raw(d, (ph, pw), float(cm), self._ray_dev, self.image_height,
                                             self.image_width, v, float(self.cuboid_side), scratch, dst_bf16, pg.lay_in,
@@ -404,7 +536,8 @@ class VoxelNetwork_depth(nn.Module):
             launches += 1
         return launches
 
-    def forward(self, images, grid_coord_proj_batch, coord_volumes, scene_volumes=None, depth_map_batch=None):
+    def forward(self, images, grid_coord_proj_batch, coord_volumes, scene_volumes=None, depth_map_batch=None,
+                camera_ids=None):
         if self.backbone_handoff:
             # SURVEY section 8f row 1: the backbone stops before its last deconvolution stage; that stage, its
             # BatchNorm + ReLU and process_features[0] run as ONE tcgen05 kernel that emits the stage's channel-last
@@ -415,9 +548,9 @@ class VoxelNetwork_depth(nn.Module):
             w, bias = self._handoff_weights(x2.device)
             return self._lift_feat32(lambda out: _lib.backbone_handoff(x2, w, bias, out=out), x2.shape[0],
                                      (2 * x2.shape[2], 2 * x2.shape[3]), x2.device, 2, grid_coord_proj_batch,
-                                     coord_volumes, scene_volumes, depth_map_batch)
+                                     coord_volumes, scene_volumes, depth_map_batch, camera_ids)
         heatmaps, features = self.backbone(images)
-        return self.lift(features, grid_coord_proj_batch, coord_volumes, scene_volumes, depth_map_batch)
+        return self.lift(features, grid_coord_proj_batch, coord_volumes, scene_volumes, depth_map_batch, camera_ids)
 
     def _handoff_weights(self, device):
         """Packed weights of the hand-off kernel, rebuilt when one of their sources changed (in-place edits bump

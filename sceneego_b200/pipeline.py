@@ -70,8 +70,12 @@ class HostStagePipeline:
         self.h2d_bytes += feat.numel() * 4 + depth.numel() * 4
         return parts
 
-    def run(self, batches: Iterable[Tuple[torch.Tensor, torch.Tensor]]) -> List[torch.Tensor]:
+    def run(self, batches: Iterable[Tuple]) -> List[torch.Tensor]:
+        """batches: (feat, depth) pinned host tensors, or (feat, depth, camera_ids) with the host-side camera ids
+        `lift` takes (a camera per frame)."""
         batches = list(batches)
+        cam_ids = [b[2] if len(b) > 2 else None for b in batches]
+        batches = [b[:2] for b in batches]
         out = []
         main = torch.cuda.current_stream(self.device)
         # pinned result buffers for every batch of this call BEFORE any GPU work is queued: cudaHostAlloc
@@ -97,13 +101,14 @@ class HostStagePipeline:
                     kps = []
                     for s0, s1, ev in ramp:
                         main.wait_event(ev)
+                        ids = None if cam_ids[0] is None else cam_ids[0][s0:s1]
                         kps.append(self.net.lift(feat[s0:s1], self.net.grid_coord_proj_batch, self.net.coord_volumes,
-                                                 depth_map_batch=depth[s0:s1])[0])
+                                                 depth_map_batch=depth[s0:s1], camera_ids=ids)[0])
                     kp = torch.cat(kps)
                 else:
                     main.wait_event(self.ready[slot])
                     kp = self.net.lift(feat, self.net.grid_coord_proj_batch, self.net.coord_volumes,
-                                       depth_map_batch=depth)[0]
+                                       depth_map_batch=depth, camera_ids=cam_ids[i])[0]
             self.done[slot].record(main)
             if self.gather_fn is not None:
                 local_kps.append(kp)
